@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                      # our CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W     # CPU reference arm
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's outputs as DIR/*.npy
 
 A "step" = one forward pass over one batch of synthetic clips of the workload's shape
 (default workload: BASELINE.json configs[2], X3D-M 10-view eval at 16x256x256, bf16,
@@ -40,6 +41,7 @@ WORKLOADS = {
     "train_m224": ("X3D_M", 16, 224, 1, 32, "float32"),     # configs[4]: one training step
 }
 METRIC = "X3D-M clips/sec"
+DUMP_LIMIT_BYTES = 64 << 20      # --dump-outputs writes at most this much
 FFMA2_PEAK_TMACS = 34.9          # measured packed-FFMA2 rate of this part, profiles/r01_microbench_fma_copy.txt
 
 
@@ -295,9 +297,24 @@ def kernel_traffic(kernel: str, workload: str, clips: int):
     return None, "no capture for this kernel/workload"
 
 
-def measure_forward(workload, clips, steps, warmup, device, world, rank, want_model=False):
+def dump_outputs(outdir, arrays):
+    """Writes each array as `outdir/<name>.npy` in float32, so that two builds can be compared output
+    for output on the same seeded inputs."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total / 2**20:.1f} MB "
+                         f"(limit {DUMP_LIMIT_BYTES >> 20} MB): lower --clips")
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
+def measure_forward(workload, clips, steps, warmup, device, world, rank, want_model=False, want_outputs=False):
     """Device-resident throughput of one forward workload (CUDA-graph replays on the captured
-    input buffer, CUDA events, max over ranks) + per-kernel-class attribution of one eager pass."""
+    input buffer, CUDA events, max over ranks) + per-kernel-class attribution of one eager pass.
+    `want_outputs`: res["outputs"] holds what the last timed step returned (probabilities, and the
+    logits the model exposes as `last_logits`), copied to the host after the timed region."""
     from x3d_tf_b200 import ops
     variant, T, S, views, dclips, dtype_name = WORKLOADS[workload]
     clips = clips or dclips
@@ -325,6 +342,9 @@ def measure_forward(workload, clips, steps, warmup, device, world, rank, want_mo
     clocks = sampler.finish()
     ms_max = _max_over_ranks(e0.elapsed_time(e1), device, world)
     value = clips * world * steps / (ms_max / 1e3)
+    # the graph's output buffers: copied now, before any later pass can overwrite them
+    outputs = {"probs": probs.float().cpu().numpy(),
+               "logits": model.last_logits.float().cpu().numpy()} if want_outputs else None
 
     # ---- per-class attribution: one eager, event-bracketed pass over the same batch
     model._use_graph = False
@@ -396,7 +416,8 @@ def measure_forward(workload, clips, steps, warmup, device, world, rank, want_mo
            "steps": steps, "clocks": clocks, "launches_per_step": len(recs), "roofline": roofline,
            "classes": classes,
            "whole_model_hbm_frac_layerwise": total_bytes / (ms_max / steps * 1e-3) / 1e9 / hbm,
-           "pointwise_tensor_pipe_util": (2 * pw_macs / (pw_ms * 1e-3) / 1e12 / tflops) if pw_ms else None}
+           "pointwise_tensor_pipe_util": (2 * pw_macs / (pw_ms * 1e-3) / 1e12 / tflops) if pw_ms else None,
+           "outputs": outputs}
     if want_model:
         res.update(model=model, static_in=static_in, probs=probs, cfg=cfg)
     return res
@@ -428,7 +449,10 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=device)
     warmup = max(args.warmup, 3)               # the contract's minimum; the line reports what ran
 
-    r = measure_forward(args.workload, args.clips, args.steps, warmup, device, world, rank, want_model=True)
+    r = measure_forward(args.workload, args.clips, args.steps, warmup, device, world, rank, want_model=True,
+                        want_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"])
     model, static_in, probs, cfg = r.pop("model"), r.pop("static_in"), r.pop("probs"), r.pop("cfg")
     clips, T, S, views, tdt, esize = r["clips"], r["T"], r["S"], r["views"], r["tdt"], r["esize"]
     extra = {"whole_model_hbm_frac_layerwise": r["whole_model_hbm_frac_layerwise"],
@@ -524,10 +548,11 @@ def run_b200(args):
         dist.destroy_process_group()
 
 
-def measure_train(workload, clips, steps, warmup, device, world, rank):
+def measure_train(workload, clips, steps, warmup, device, world, rank, want_outputs=False):
     """BASELINE configs[4]: one X3D-M training step (forward, backward, NCCL gradient all-reduce,
     SGD-Nesterov) per bench step; batch 32 per GPU, 16x224x224, fp32 (the reference's default
-    precision; train.py:85-152).  value = clips trained per second over all ranks."""
+    precision; train.py:85-152).  value = clips trained per second over all ranks.
+    `want_outputs`: res["outputs"] holds the per-clip losses the last timed step returned."""
     import torch.distributed as dist
     from x3d_tf_b200 import _lib
     from x3d_tf_b200.arch import build_arch
@@ -562,6 +587,7 @@ def measure_train(workload, clips, steps, warmup, device, world, rank):
     launches = _lib.calls - c0
     ms_max = _max_over_ranks(e0.elapsed_time(e1), device, world)
     value = clips * world * steps / (ms_max / 1e3)
+    outputs = {"loss": loss.float().cpu().numpy()} if want_outputs else None
 
     # the exchange step alone: the same flat fp32 gradient arena, summed over the ranks
     ar_ms = 0.0
@@ -606,7 +632,7 @@ def measure_train(workload, clips, steps, warmup, device, world, rank):
                    "d2h_bytes_per_step": host_loss.numel() * 4, "steps": n_e2e,
                    "api": "X3DTrainer.step on clips/labels copied from pinned host memory, per-clip losses read back"},
            "momentum": tr.momentum, "dropout": tr.dropout, "x_bytes": x.numel() * 4,
-           "loss_mean": float(loss.float().mean().item())}
+           "loss_mean": float(loss.float().mean().item()), "outputs": outputs}
     del tr, x, host_x
     torch.cuda.empty_cache()
     return res
@@ -623,7 +649,10 @@ def run_train(args):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=device)
     warmup = max(args.warmup, 3)
-    r = measure_train(args.workload, args.clips, args.steps, warmup, device, world, rank)
+    r = measure_train(args.workload, args.clips, args.steps, warmup, device, world, rank,
+                      want_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"])
     if rank == 0:
         line = {"metric": "X3D-M training clips/sec", "value": r["value"], "unit": "clips/s", "n_gpus": world,
                 "steps": args.steps, "warmup": warmup, "ms_per_step": r["ms_per_step"],
@@ -660,7 +689,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` array (the other BASELINE configs)")
     ap.add_argument("--config-steps", type=int, default=10, help="timed steps of each `configs` entry (>= 10)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none to write")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload.startswith("train"):
