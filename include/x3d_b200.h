@@ -250,6 +250,25 @@ int x3d_normalize_u8(const uint8_t* in, void* out, int64_t pixels, const float* 
  * to the model:   video [F,H,W,3] uint8 -> out [crops*views, T, S, S, 3] uint8 (crop-major). */
 int x3d_eval_views_u8(const uint8_t* video, uint8_t* out, int F, int H, int W, int T, int views,
                       int crops, int S, void* stream);
+/* Clips of decoded videos of any resolution (transforms.py:112-147, 192-227): per clip a bilinear
+ * short-side resize of every source frame to rh x rw (tf.image.resize bilinear = TF 2.4
+ * ResizeBilinear with half_pixel_centers, fp32 with every operation rounded separately, then a
+ * truncating cast to uint8), an S x S crop at (y0, x0) of the resized frame and, for flip = 1, a
+ * left-right flip of the crop:
+ *   out[n][t][y][x][c] = resized(frame n,t)[y0 + y][x0 + (flip ? S-1-x : x)][c]
+ *   frames     packed uint8 frames [*, H, W, 3] of a ragged batch of videos (device);
+ *   frame_off  int64 [N*T] (device): byte offset in `frames` of the source frame of output frame (n, t);
+ *   desc       x3d_clip_desc [N] (device): the source extent H x W, resized extent rh x rw, crop
+ *              origin and flip of clip n;
+ *   out        [N, T, S, S, 3] uint8 (4-byte aligned).
+ * The descriptors are device data and are NOT checked by the call; the caller guarantees, per clip:
+ * H, W >= 1; S <= rh, S <= rw; 0 <= y0 <= rh - S; 0 <= x0 <= rw - S; flip in {0, 1}; every frame
+ * frame_off[n*T+t] .. + H*W*3 inside `frames`.  S <= 2048.  One launch covers the whole batch, so
+ * every video can have its own frame count and frame size.  x3d_eval_views_u8 is this kernel over a
+ * plan passed by value (rh = H, rw = W: an identity resize, which is exact). */
+typedef struct x3d_clip_desc { int32_t H, W, rh, rw, y0, x0, flip; } x3d_clip_desc;
+int x3d_video_clips_u8(const uint8_t* frames, const int64_t* frame_off, const x3d_clip_desc* desc, int N,
+                       int T, int S, uint8_t* out, void* stream);
 /* x3d_stem_tc_fwd with the input stage fused into its loader: uint8 NDHWC clips in, bf16
  * activations out (same result as x3d_normalize_u8(bf16) followed by x3d_stem_tc_fwd). */
 int x3d_stem_tc_u8_fwd(const uint8_t* in, const float* mean, const float* std, float norm_value,

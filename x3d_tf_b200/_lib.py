@@ -41,6 +41,11 @@ class PwTcArgs(C.Structure):
                 ("colmean", C.c_void_p), ("store_d", C.c_int32), ("reserved", C.c_int32)]
 
 
+class ClipDesc(C.Structure):
+    _fields_ = [("H", C.c_int32), ("W", C.c_int32), ("rh", C.c_int32), ("rw", C.c_int32),
+                ("y0", C.c_int32), ("x0", C.c_int32), ("flip", C.c_int32)]
+
+
 # name -> (restype, argtypes); must list every symbol include/x3d_b200.h declares.
 SIGNATURES = {
     "x3d_version": (C.c_int, []),
@@ -105,6 +110,7 @@ SIGNATURES = {
     "x3d_normalize_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_float),
                                    C.POINTER(C.c_float), C.c_float, C.c_int, C.c_void_p]),
     "x3d_eval_views_u8": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 7 + [C.c_void_p]),
+    "x3d_video_clips_u8": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p, C.c_void_p]),
     "x3d_stem_tc_u8_fwd": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_float,
                                      C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p]),
     "x3d_eval_metrics": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,

@@ -13,8 +13,11 @@ every batch, `utils.py:160-167`), the four metric sums are all-reduced at the en
 Video decoding (`dataloader.py`, `transforms.py`) is outside this path.  `--test_file_pattern`
 names a text file with one `<path> <label>` line per video as in the reference, where <path> is
 a `.npy` file of already decoded and cropped uint8 clips `[num_preds, T, H, W, 3]` (normalised on
-the device, `utils.py:42-72`) or float32 clips (already normalised).  `--synthetic V` evaluates V
-seeded random videos instead (no files needed).
+the device, `utils.py:42-72`) or float32 clips (already normalised).  With `--decoded_videos` the
+lines name decoded videos `[F, H, W, 3]` uint8 of any frame count and size instead: the short-side
+resize, temporal views and crops of `transforms.py` run on the device (`video.py`,
+x3d_video_clips_u8), and only the frames the views sample are read and copied.  `--synthetic V`
+evaluates V seeded random videos instead (no files needed).
 """
 from __future__ import annotations
 
@@ -63,6 +66,15 @@ def file_batches(items: List[Tuple[str, int]], videos_per_batch: int, num_preds:
         yield np.concatenate(clips, 0), np.asarray([lab for _, lab in chunk], np.int32)
 
 
+def video_batches(items: List[Tuple[str, int]], videos_per_batch: int, cfg):
+    """Batches of decoded videos (`.npy` [F, H, W, 3] uint8, memory-mapped) as video.VideoBatch."""
+    from . import video
+    for i in range(0, len(items), videos_per_batch):
+        chunk = items[i:i + videos_per_batch]
+        yield (video.eval_batch([video.load_video(p) for p, _ in chunk], cfg),
+               np.asarray([lab for _, lab in chunk], np.int32))
+
+
 def synthetic_batches(lo: int, hi: int, videos_per_batch: int, num_preds: int, T: int, S: int,
                       num_classes: int) -> Iterator[Tuple[np.ndarray, np.ndarray]]:
     """Seeded per VIDEO (not per rank), so any sharding evaluates the same set."""
@@ -88,6 +100,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     ap.add_argument("--cfg", required=True, help="config .yaml (reference layout) or a variant name, e.g. X3D_M")
     ap.add_argument("--test_file_pattern", default=None, help="text file: '<clips.npy> <label>' per video")
     ap.add_argument("--model_folder", required=True, help="directory with a TF `checkpoint` file")
+    ap.add_argument("--decoded_videos", action="store_true",
+                    help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--synthetic", type=int, default=0, help="evaluate this many seeded random videos")
     ap.add_argument("--dtype", default=None, choices=["bfloat16", "float32"],
@@ -140,7 +154,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     else:
         items = read_file_list(a.test_file_pattern)
         lo, hi = shard.shard_range(len(items), world, rank)
-        data = file_batches(items[lo:hi], vpb, num_preds)
+        data = (video_batches(items[lo:hi], vpb, cfg) if a.decoded_videos
+                else file_batches(items[lo:hi], vpb, num_preds))
     res = model.evaluate(data, verbose=1 if rank == 0 else 0)
     if rank == 0:
         print(f"\nloss: {res['loss']:.4f} - acc: {res['acc']:.4f} - top_5_acc: {res['top_5_acc']:.4f} "

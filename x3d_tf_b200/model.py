@@ -24,6 +24,7 @@ import torch
 from . import arch as A
 from . import ops
 from . import tf_bundle
+from .video import VideoBatch
 
 _BN_LEAVES = ("gamma", "beta", "moving_mean", "moving_variance")
 
@@ -879,7 +880,8 @@ class X3D(Layer):
             lr_schedule=None, verbose: int = 0, **_):
         """Keras `model.fit` as train.py:145-152 uses it: for every epoch the learning rate comes from
         `lr_schedule(epoch)` (train.py:114-125, default training.lr_schedule of this model's cfg),
-        `steps_per_epoch` batches `(clips, labels)` are taken from `dataset` (re-iterated per epoch),
+        `steps_per_epoch` batches `(clips, labels)` are taken from `dataset` (re-iterated per epoch; clips
+        as for `call`, or a video.VideoBatch whose clips are built on the device),
         each one forward + backward + gradient all-reduce over the initialised torch.distributed
         group + optimizer step (cfg.TRAIN.OPTIMIZER).  Returns {"loss": [per-epoch mean]}.  The model's
         variables hold the trained values afterwards (call / evaluate / save_weights see them)."""
@@ -896,7 +898,7 @@ class X3D(Layer):
             for i, (clips, labels) in enumerate(dataset):
                 if steps_per_epoch is not None and i >= steps_per_epoch:
                     break
-                x = _as_device_clip(clips, dev)
+                x = clips.clips(dev) if isinstance(clips, VideoBatch) else _as_device_clip(clips, dev)
                 if x.dtype == torch.uint8:
                     x = ops.normalize_u8(x, mean, std, torch.float32)
                 lab = torch.as_tensor(np.asarray(labels.cpu() if isinstance(labels, torch.Tensor) else labels)
@@ -970,7 +972,9 @@ class X3D(Layer):
         [videos, classes] in order.  uint8 batches are normalised on the device (fused into the
         stem's loader in bf16 mode).  `on_device(probs, i)`, if given, is called right after the
         replay of batch i with the device-resident probabilities (stream-ordered: enqueue work on
-        the current stream, do not keep the tensor)."""
+        the current stream, do not keep the tensor).  A batch can also be a video.VideoBatch: its
+        packed decoded frames are copied on the copy stream and x3d_video_clips_u8 builds the uint8
+        clips on that stream directly in the graph's input buffer."""
         self._no_training(training)
         if not torch.cuda.is_available():
             raise RuntimeError("no CUDA device: the X3D path has no CPU implementation")
@@ -982,6 +986,8 @@ class X3D(Layer):
         slots: Dict[tuple, dict] = {}
 
         def stage(hb, slot):
+            if isinstance(hb, VideoBatch):
+                return stage_video(hb, slot)
             if isinstance(hb, np.ndarray):
                 hb = torch.from_numpy(np.ascontiguousarray(hb))
             if hb.dtype in (torch.float16, torch.float64):
@@ -997,6 +1003,33 @@ class X3D(Layer):
             st["used"] = True
             with torch.cuda.stream(cs):
                 static_in.copy_(hb, non_blocking=True)
+                st["copied"].record(cs)
+            return st
+
+        def stage_video(vb, slot):
+            # the packed frames go to this slot's own staging buffer on the copy stream, and the clip
+            # kernel runs on that stream straight into the graph's uint8 input: `done` (the replay that
+            # last read the slot) orders both buffers, `copied` orders the replay behind the kernel
+            self._check_input(vb.shape)
+            g, static_in, s_probs, s_logits = self._graph(vb.shape, torch.uint8, device, slot, training)
+            st = slots.setdefault((tuple(vb.shape), torch.uint8, slot), {
+                "host_out": torch.empty(tuple(s_probs.shape), dtype=torch.float32).pin_memory(),
+                "done": torch.cuda.Event(), "copied": torch.cuda.Event()})
+            st.update(g=g, s_probs=s_probs, s_logits=s_logits)
+            cs.wait_event(st["done"])
+            cs.wait_stream(main) if not st.get("used") else None
+            st["used"] = True
+            nbytes = vb.frames.numel()
+            with torch.cuda.stream(cs):
+                if st.get("frames") is None or st["frames"].numel() < nbytes:
+                    st["frames"] = torch.empty(nbytes, dtype=torch.uint8, device=device)
+                    st["frame_off"] = torch.empty(vb.frame_off.shape, dtype=torch.int64, device=device)
+                    st["desc"] = torch.empty(vb.desc.shape, dtype=torch.int32, device=device)
+                frames = st["frames"][:nbytes]
+                frames.copy_(vb.frames, non_blocking=True)
+                st["frame_off"].copy_(vb.frame_off, non_blocking=True)
+                st["desc"].copy_(vb.desc, non_blocking=True)
+                ops.video_clips_u8(frames, st["frame_off"], st["desc"], vb.shape[1], vb.shape[2], out=static_in)
                 st["copied"].record(cs)
             return st
 

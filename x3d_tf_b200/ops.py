@@ -136,6 +136,29 @@ def eval_views_u8(video: torch.Tensor, T: int, views: int, crops: int, size: int
     return out
 
 
+def video_clips_u8(frames: torch.Tensor, frame_off: torch.Tensor, desc: torch.Tensor, T: int, S: int,
+                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Clips of a ragged batch of decoded videos (device): per clip a bilinear short-side resize, an
+    S x S crop and a flip, as x3d_video_clips_u8 describes.  `frames` packed uint8 frames, `frame_off`
+    int64 [N*T] byte offsets of each output frame's source, `desc` int32 [N, 7] x3d_clip_desc rows
+    (validated on the host: video.validate) -> [N, T, S, S, 3] uint8 (written into `out` if given)."""
+    for t, name in ((frames, "frames"), (frame_off, "frame_off"), (desc, "desc")):
+        _req(t, name)
+    if frames.dtype != torch.uint8 or frame_off.dtype != torch.int64 or desc.dtype != torch.int32:
+        raise TypeError("video_clips_u8: frames uint8, frame_off int64, desc int32")
+    N = desc.shape[0]
+    if desc.dim() != 2 or desc.shape[1] != 7 or frame_off.numel() != N * T:
+        raise ValueError(f"video_clips_u8: desc {tuple(desc.shape)} / frame_off {frame_off.numel()} for T={T}")
+    shape = (N, T, S, S, 3)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=frames.device)
+    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous():
+        raise ValueError(f"video_clips_u8: out must be contiguous uint8 {shape}")
+    _launch("x3d_video_clips_u8", lambda: lib().x3d_video_clips_u8(
+        frames.data_ptr(), frame_off.data_ptr(), desc.data_ptr(), N, T, S, out.data_ptr(), _stream()))
+    return out
+
+
 def stem_tc_u8_fwd(x: torch.Tensor, mean, std, wc: torch.Tensor, bias: torch.Tensor,
                    norm_value: float = 255.0) -> torch.Tensor:
     """Tensor-core stem with the uint8 input stage fused into its loader; bf16 activations out."""

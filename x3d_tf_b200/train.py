@@ -15,7 +15,10 @@ MirroredStrategy does (`utils.py:160-167`); gradients are summed by one NCCL all
 
 Out of scope here as in eval.py's driver: video decoding and augmentation (`dataloader.py`,
 `transforms.py`).  File lists name `.npy` arrays of already decoded and cropped uint8 clips
-`[T, H, W, 3]` (or `[k, T, H, W, 3]`: k training clips of one video) with an integer label;
+`[T, H, W, 3]` (or `[k, T, H, W, 3]`: k training clips of one video) with an integer label, or,
+with `--decoded_videos`, decoded videos `[F, H, W, 3]` uint8 of any size: then every global-batch
+slot draws one random clip of its video (temporal start, short-side scale jitter, crop, flip;
+`video.train_plan`) and the resize / crop / flip run on the device (x3d_video_clips_u8);
 `--synthetic N` trains on N seeded random clips per epoch instead.  W&B / TensorBoard callbacks are
 not reproduced; the per-epoch log line carries the same quantities Keras prints.
 """
@@ -79,6 +82,19 @@ def file_clip_batches(items: List[Tuple[str, int]], gbatch: int, steps: int, see
         yield np.stack(clips), np.asarray(labels, np.int32)
 
 
+def video_clip_batches(items: List[Tuple[str, int]], gbatch: int, steps: int, seed: int, cfg, rank: int = 0,
+                       world: int = 1, crop_size: int = 0):
+    """This rank's slice of every global batch as a video.VideoBatch: one random clip per listed
+    decoded video, the random numbers from video.train_rng(seed, rank) (per epoch and rank)."""
+    from . import video
+    batch = gbatch // world
+    rng = video.train_rng(seed, rank)
+    for idx in global_batch_indices(len(items), gbatch, steps, seed):
+        mine = idx[rank * batch:(rank + 1) * batch]
+        vb = video.train_batch([video.load_video(items[j][0]) for j in mine], cfg, rng, crop_size)
+        yield vb, np.asarray([items[j][1] for j in mine], np.int32)
+
+
 def synthetic_clip_batches(steps: int, batch: int, T: int, S: int, num_classes: int, seed: int
                            ) -> Iterator[Tuple[np.ndarray, np.ndarray]]:
     rng = np.random.default_rng(seed)
@@ -92,6 +108,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     ap.add_argument("--config", required=True, help="config .yaml (reference layout) or a variant name")
     ap.add_argument("--train_file_pattern", default=None)
     ap.add_argument("--val_file_pattern", default=None)
+    ap.add_argument("--decoded_videos", action="store_true",
+                    help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
     ap.add_argument("--model_dir", required=True)
     ap.add_argument("--pretrained_ckpt", default=None)
     ap.add_argument("--num_gpus", type=int, default=1)
@@ -133,7 +151,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     from .arch import build_arch
     from .model import X3D, keras_default_weights, reset_block_counters
     from .training import X3DTrainer
-    from .eval import file_batches
+    from .eval import file_batches, video_batches
+    from .video import VideoBatch
 
     tr = X3DTrainer(cfg, device=dev, world=world, rank=rank)
     # a from-scratch run starts where `X3D(cfg)` starts in the reference (train.py:128): Keras default
@@ -169,12 +188,15 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
         if rank == 0:
             print(f"\nEpoch {epoch + 1}/{epochs}\nEpoch {epoch + 1:05d}: LearningRateScheduler setting learning rate to {lr}.")
         # every rank runs exactly `steps` steps (rank-independent count; short lists repeat)
-        data = (file_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, rank, world) if items is not None
-                else synthetic_clip_batches(steps, batch, T, S, cfg.NETWORK.NUM_CLASSES,
-                                            1111 + 7919 * epoch + rank))
+        if items is not None and a.decoded_videos:
+            data = video_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size)
+        else:
+            data = (file_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, rank, world) if items is not None
+                    else synthetic_clip_batches(steps, batch, T, S, cfg.NETWORK.NUM_CLASSES,
+                                                1111 + 7919 * epoch + rank))
         t0, n, loss_sum = time.time(), 0, torch.zeros((), dtype=torch.float64, device=dev)
         for clips, labels in data:
-            x = torch.from_numpy(clips).to(dev, non_blocking=True)
+            x = clips.clips(dev) if isinstance(clips, VideoBatch) else torch.from_numpy(clips).to(dev, non_blocking=True)
             if x.dtype == torch.uint8:
                 x = ops.normalize_u8(x, mean, std, torch.float32)           # utils.normalize on the device
             loss = tr.step(x.float(), torch.from_numpy(labels).to(dev), lr)
@@ -196,7 +218,9 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
             num_preds = cfg.TEST.NUM_TEMPORAL_VIEWS * cfg.TEST.NUM_SPATIAL_CROPS
             from .shard import shard_range
             lo, hi = shard_range(len(val_items), world, rank)
-            res = m.evaluate(file_batches(val_items[lo:hi], max(cfg.TEST.BATCH_SIZE // num_preds, 1), num_preds))
+            vpb = max(cfg.TEST.BATCH_SIZE // num_preds, 1)
+            res = m.evaluate(video_batches(val_items[lo:hi], vpb, cfg) if a.decoded_videos
+                             else file_batches(val_items[lo:hi], vpb, num_preds))
             log.update(val_loss=res["loss"], val_acc=res["acc"], val_top_5_acc=res["top_5_acc"])
             del m
         if rank == 0:
