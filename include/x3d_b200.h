@@ -269,6 +269,85 @@ int x3d_eval_views_u8(const uint8_t* video, uint8_t* out, int F, int H, int W, i
 typedef struct x3d_clip_desc { int32_t H, W, rh, rw, y0, x0, flip; } x3d_clip_desc;
 int x3d_video_clips_u8(const uint8_t* frames, const int64_t* frame_off, const x3d_clip_desc* desc, int N,
                        int T, int S, uint8_t* out, void* stream);
+/* ---- Baseline JPEG decoding of the frames of TFRecord videos ------------------------------------
+ * The reference reads GZIP TFRecords of SequenceExamples whose frames are JPEG images and decodes them
+ * with tf.io.decode_jpeg (dataloader.py:66-91, 150-174; eval.py --tfrecord, train.py --use_tfrecord).
+ * These three stages reproduce libjpeg-turbo's decompressor in its default libjpeg-6b mode (what TF 2.4
+ * and Pillow link) bit for bit, for baseline sequential Huffman, 8-bit, three components in one
+ * interleaved scan, luma sampling 2x2 or 1x1, chroma 1x1, no restart interval (x3d_tf_b200/jpeg.py
+ * parses the headers and rejects everything else on the host).  Every frame of a ragged batch is
+ * decoded by one launch per stage.
+ *
+ * Per frame (component c = 0 luma, 1 Cb, 2 Cr; hs = vs = luma sampling, 1 for chroma):
+ *   mcux = ceil(W / (8*hs)), mcuy = ceil(H / (8*vs));  component c has a block grid of
+ *   bw_c x bh_c = (mcux*hs_c) x (mcuy*vs_c) blocks, stored component after component, each row-major:
+ *   coefficients  int16 [blocks][64], natural order, quantised;  block b of the frame at
+ *                 coef + (coef_off + b) * 64.  blocks = sum_c bw_c * bh_c.
+ *   planes        uint8, plane c = [bh_c*8][bw_c*8] samples at plane_off + sum_{c'<c} bw_c'*bh_c'*64.
+ *   output        packed row-major [H][W][3] RGB at out_off (4-byte aligned): exactly what
+ *                 x3d_video_clips_u8 reads through frame_off.
+ * The descriptors are device data and are NOT checked by the calls; the caller guarantees per frame:
+ * 1 <= H, W <= 65535; (hs, vs) = (1, 1) or (2, 2); 0 <= tables < the number of table sets; the segment
+ * seg_off .. + seg_len inside `data`; every buffer range above inside its buffer; status < the length
+ * of `status`.  Ranges of different frames may not overlap. */
+typedef struct x3d_jpeg_frame {
+  int64_t seg_off;     /* byte offset in `data` of the entropy-coded segment (byte stuffing included) */
+  int64_t coef_off;    /* first coefficient block */
+  int64_t plane_off;   /* first byte of the sample planes */
+  int64_t out_off;     /* first byte of the RGB output (multiple of 4) */
+  int32_t seg_len;     /* bytes of the segment, up to (not including) the marker that ends it */
+  int32_t H, W;
+  int32_t hs, vs;      /* luma sampling factors */
+  int32_t tables;      /* index of its x3d_jpeg_tables */
+  int32_t status;      /* index of its status word */
+  int32_t reserved;
+} x3d_jpeg_frame;
+/* One Huffman table as libjpeg's jpeg_make_d_derived_tbl derives it (jdhuff.c):
+ *   maxcode[l]   largest code of length l (1..16), -1 if none; maxcode[17] = 0xFFFFF
+ *   valoffset[l] huffval index of the first code of length l minus that code
+ *   lookup[b]    for the next 8 bits b: (length << 8) | symbol of the code they start with, or 9 << 8
+ *                when that code is longer than 8 bits */
+typedef struct x3d_jpeg_huff {
+  int32_t maxcode[18];
+  int32_t valoffset[18];
+  uint16_t lookup[256];
+  uint8_t huffval[256];
+} x3d_jpeg_huff;
+/* The tables of one header (frames of one encoder run share it): quantisation tables in natural order
+ * by table id, the derived DC / AC Huffman tables by table id, and which of them each component uses. */
+typedef struct x3d_jpeg_tables {
+  x3d_jpeg_huff dc[2];
+  x3d_jpeg_huff ac[2];
+  uint16_t q[4][64];
+  int32_t comp_q[3], comp_dc[3], comp_ac[3];
+  int32_t reserved;
+} x3d_jpeg_tables;
+enum x3d_jpeg_status {
+  X3D_JPEG_OK = 0,
+  X3D_JPEG_BAD_CODE = 1,       /* no Huffman code of length <= 16 matches */
+  X3D_JPEG_BAD_RUN = 2,        /* a run of zeros or a coefficient past coefficient 63 */
+  X3D_JPEG_SHORT_DATA = 3      /* the segment ended before the last block (libjpeg reads zeros there) */
+};
+enum x3d_jpeg_dct { X3D_JPEG_ISLOW = 0, X3D_JPEG_IFAST = 1 };
+/* Stage 1, Huffman decoding (jdhuff.c decode_mcu): one warp per frame.  Writes every coefficient block
+ * of the frame (zeros where no coefficient is coded) and status[frame.status] (x3d_jpeg_status); after
+ * an error the remaining blocks of that frame are left as they were.  Never reads outside the frame's
+ * segment or writes outside its blocks. */
+int x3d_jpeg_entropy(const uint8_t* data, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,
+                     int nframes, int16_t* coef, int32_t* status, void* stream);
+/* Stage 2, dequantisation and 8x8 inverse DCT into the planes: method X3D_JPEG_ISLOW = jidctint.c
+ * jpeg_idct_islow, X3D_JPEG_IFAST = jidctfst.c jpeg_idct_ifast with jddctmgr.c's multiplier table
+ * (q * aanscales, descaled by 12 with rounding); both with IDCT_range_limit (wrap-around at RANGE_MASK).
+ * max_blocks >= the block count of every frame. */
+int x3d_jpeg_idct(const int16_t* coef, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,
+                  int nframes, int max_blocks, int method, uint8_t* planes, void* stream);
+/* Stage 3, upsampling and colour conversion into the output: chroma of 2x2 frames by jdsample.c
+ * h2v2_fancy_upsample (edges replicated at the downsampled extent ceil(W/2) x ceil(H/2); the box
+ * h2v2_upsample when ceil(W/2) <= 2, as libjpeg does), then jdcolor.c ycc_rgb_convert.
+ * max_pixels >= H*W of every frame. */
+int x3d_jpeg_color(const uint8_t* planes, const x3d_jpeg_frame* frames, int nframes, int64_t max_pixels,
+                   uint8_t* out, void* stream);
+
 /* x3d_stem_tc_fwd with the input stage fused into its loader: uint8 NDHWC clips in, bf16
  * activations out (same result as x3d_normalize_u8(bf16) followed by x3d_stem_tc_fwd). */
 int x3d_stem_tc_u8_fwd(const uint8_t* in, const float* mean, const float* std, float norm_value,

@@ -46,6 +46,25 @@ class ClipDesc(C.Structure):
                 ("y0", C.c_int32), ("x0", C.c_int32), ("flip", C.c_int32)]
 
 
+class JpegFrame(C.Structure):
+    _fields_ = [("seg_off", C.c_int64), ("coef_off", C.c_int64), ("plane_off", C.c_int64), ("out_off", C.c_int64),
+                ("seg_len", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("hs", C.c_int32), ("vs", C.c_int32),
+                ("tables", C.c_int32), ("status", C.c_int32), ("reserved", C.c_int32)]
+
+
+class JpegHuff(C.Structure):
+    _fields_ = [("maxcode", C.c_int32 * 18), ("valoffset", C.c_int32 * 18), ("lookup", C.c_uint16 * 256),
+                ("huffval", C.c_uint8 * 256)]
+
+
+class JpegTables(C.Structure):
+    _fields_ = [("dc", JpegHuff * 2), ("ac", JpegHuff * 2), ("q", (C.c_uint16 * 64) * 4),
+                ("comp_q", C.c_int32 * 3), ("comp_dc", C.c_int32 * 3), ("comp_ac", C.c_int32 * 3),
+                ("reserved", C.c_int32)]
+
+
+X3D_JPEG_ISLOW, X3D_JPEG_IFAST = 0, 1
+
 # name -> (restype, argtypes); must list every symbol include/x3d_b200.h declares.
 SIGNATURES = {
     "x3d_version": (C.c_int, []),
@@ -111,6 +130,9 @@ SIGNATURES = {
                                    C.POINTER(C.c_float), C.c_float, C.c_int, C.c_void_p]),
     "x3d_eval_views_u8": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 7 + [C.c_void_p]),
     "x3d_video_clips_u8": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p, C.c_void_p]),
+    "x3d_jpeg_entropy": (C.c_int, [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3),
+    "x3d_jpeg_idct": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p] * 2),
+    "x3d_jpeg_color": (C.c_int, [C.c_void_p] * 2 + [C.c_int, C.c_int64] + [C.c_void_p] * 2),
     "x3d_stem_tc_u8_fwd": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_float,
                                      C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p]),
     "x3d_eval_metrics": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,

@@ -16,12 +16,18 @@ a `.npy` file of already decoded and cropped uint8 clips `[num_preds, T, H, W, 3
 the device, `utils.py:42-72`) or float32 clips (already normalised).  With `--decoded_videos` the
 lines name decoded videos `[F, H, W, 3]` uint8 of any frame count and size instead: the short-side
 resize, temporal views and crops of `transforms.py` run on the device (`video.py`,
-x3d_video_clips_u8), and only the frames the views sample are read and copied.  `--synthetic V`
-evaluates V seeded random videos instead (no files needed).
+x3d_video_clips_u8), and only the frames the views sample are read and copied.  With `--tfrecord`
+(the reference's flag) `--test_file_pattern` is a glob of the reference's GZIP TFRecord files
+(`tfrecord.py`; taken in sorted order, ranks get contiguous blocks of files, records are read in
+file order): the JPEG frames the views sample are decoded on the device (x3d_jpeg_*) and then go
+through the same clip kernel.  `--dct_method` picks the IDCT as TF's decode_jpeg names it:
+INTEGER_FAST (TF 2.4's default for dct_method='') or INTEGER_ACCURATE.  `--synthetic V` evaluates V
+seeded random videos instead (no files needed).
 """
 from __future__ import annotations
 
 import argparse
+import glob
 import os
 import sys
 from typing import Iterator, List, Optional, Tuple
@@ -75,6 +81,28 @@ def video_batches(items: List[Tuple[str, int]], videos_per_batch: int, cfg):
                np.asarray([lab for _, lab in chunk], np.int32))
 
 
+def tfrecord_files(pattern: str) -> List[str]:
+    """The GZIP TFRecord files a glob names, sorted."""
+    files = sorted(glob.glob(pattern))
+    if not files:
+        raise FileNotFoundError(f"no TFRecord files match {pattern!r}")
+    return files
+
+
+def tfrecord_batches(files: List[str], videos_per_batch: int, cfg, dct_method: str = "INTEGER_FAST"):
+    """Batches of the videos in `files` (read in file order) as video.VideoBatch of JPEG frames."""
+    from . import tfrecord, video
+    chunk = []
+    for path in files:
+        for v in tfrecord.read_videos(path):
+            chunk.append(v)
+            if len(chunk) == videos_per_batch:
+                yield video.eval_batch(chunk, cfg, dct_method), np.asarray([c.label for c in chunk], np.int32)
+                chunk = []
+    if chunk:
+        yield video.eval_batch(chunk, cfg, dct_method), np.asarray([c.label for c in chunk], np.int32)
+
+
 def synthetic_batches(lo: int, hi: int, videos_per_batch: int, num_preds: int, T: int, S: int,
                       num_classes: int) -> Iterator[Tuple[np.ndarray, np.ndarray]]:
     """Seeded per VIDEO (not per rank), so any sharding evaluates the same set."""
@@ -102,6 +130,10 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     ap.add_argument("--model_folder", required=True, help="directory with a TF `checkpoint` file")
     ap.add_argument("--decoded_videos", action="store_true",
                     help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
+    ap.add_argument("--tfrecord", action="store_true",
+                    help="--test_file_pattern is a glob of GZIP TFRecord files (JPEG frames, decoded on the device)")
+    ap.add_argument("--dct_method", default="INTEGER_FAST", choices=["INTEGER_FAST", "INTEGER_ACCURATE"],
+                    help="IDCT of the JPEG decoder (tf.io.decode_jpeg's names; INTEGER_FAST is its default)")
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--synthetic", type=int, default=0, help="evaluate this many seeded random videos")
     ap.add_argument("--dtype", default=None, choices=["bfloat16", "float32"],
@@ -114,6 +146,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     a = ap.parse_args(argv)
     if not a.test_file_pattern and not a.synthetic:
         ap.error("one of --test_file_pattern / --synthetic is required")
+    if a.tfrecord and a.decoded_videos:
+        ap.error("--tfrecord and --decoded_videos are mutually exclusive")
     cfg = load_cfg(a.cfg)
     if not os.path.isdir(a.model_folder):
         raise NotADirectoryError(a.model_folder)          # eval.py:36-37
@@ -151,6 +185,10 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
         lo, hi = shard.shard_range(a.synthetic, world, rank)
         data = synthetic_batches(lo, hi, vpb, num_preds, cfg.DATA.TEMP_DURATION, cfg.DATA.TEST_CROP_SIZE,
                                  cfg.NETWORK.NUM_CLASSES)
+    elif a.tfrecord:
+        files = tfrecord_files(a.test_file_pattern)
+        lo, hi = shard.shard_range(len(files), world, rank)
+        data = tfrecord_batches(files[lo:hi], vpb, cfg, a.dct_method)
     else:
         items = read_file_list(a.test_file_pattern)
         lo, hi = shard.shard_range(len(items), world, rank)

@@ -974,7 +974,10 @@ class X3D(Layer):
         replay of batch i with the device-resident probabilities (stream-ordered: enqueue work on
         the current stream, do not keep the tensor).  A batch can also be a video.VideoBatch: its
         packed decoded frames are copied on the copy stream and x3d_video_clips_u8 builds the uint8
-        clips on that stream directly in the graph's input buffer."""
+        clips on that stream directly in the graph's input buffer.  A VideoBatch of JPEG frames
+        (video.pack_jpeg) is decoded on the copy stream first; its status words come back with the
+        probabilities, and a corrupt frame raises ValueError naming its record and frame when that
+        batch's results are synchronised."""
         self._no_training(training)
         if not torch.cuda.is_available():
             raise RuntimeError("no CUDA device: the X3D path has no CPU implementation")
@@ -1021,17 +1024,41 @@ class X3D(Layer):
             st["used"] = True
             nbytes = vb.frames.numel()
             with torch.cuda.stream(cs):
-                if st.get("frames") is None or st["frames"].numel() < nbytes:
-                    st["frames"] = torch.empty(nbytes, dtype=torch.uint8, device=device)
+                if vb.encoded is not None:
+                    # JPEG frames: decoded on this stream into the slot's scratch (coefficients, planes,
+                    # frames); the status words come back with the probabilities and are checked when
+                    # this batch's results are synchronised
+                    frames, status = vb.encoded.decode(device, st)
+                    if st.get("host_status") is None or st["host_status"].numel() < status.numel():
+                        st["host_status"] = torch.empty(status.numel(), dtype=torch.int32).pin_memory()
+                    st["status"] = status
+                    decode_checks[batch_no[0]] = vb.encoded
+                else:
+                    if st.get("frames") is None or st["frames"].numel() < nbytes:
+                        st["frames"] = torch.empty(nbytes, dtype=torch.uint8, device=device)
+                    frames = st["frames"][:nbytes]
+                    frames.copy_(vb.frames, non_blocking=True)
+                    st["status"] = None
+                if st.get("frame_off") is None or st["frame_off"].shape != vb.frame_off.shape:
                     st["frame_off"] = torch.empty(vb.frame_off.shape, dtype=torch.int64, device=device)
                     st["desc"] = torch.empty(vb.desc.shape, dtype=torch.int32, device=device)
-                frames = st["frames"][:nbytes]
-                frames.copy_(vb.frames, non_blocking=True)
                 st["frame_off"].copy_(vb.frame_off, non_blocking=True)
                 st["desc"].copy_(vb.desc, non_blocking=True)
                 ops.video_clips_u8(frames, st["frame_off"], st["desc"], vb.shape[1], vb.shape[2], out=static_in)
                 st["copied"].record(cs)
             return st
+
+        # batch index -> EncodedFrames of a JPEG batch, then (EncodedFrames, the pinned buffer its status
+        # words were copied to): the next staging of the slot may replace the slot's buffer before the check
+        decode_checks: Dict[int, object] = {}
+        batch_no = [0]                                # index of the batch being staged
+
+        def finish(st, j):
+            st["done"].synchronize()
+            chk = decode_checks.pop(j, None)
+            if chk is not None:
+                chk[0].check(chk[1].numpy())
+            return st["host_out"].clone()
 
         it = iter(batches)
         first = next(it, None)
@@ -1041,20 +1068,23 @@ class X3D(Layer):
         while nxt is not None:
             cur = nxt
             hb = next(it, None)
+            batch_no[0] = i + 1
             nxt = stage(hb, (i + 1) & 1) if hb is not None else None
             main.wait_event(cur["copied"])
             cur["g"].replay()
             if on_device is not None:
                 on_device(cur["s_probs"], i)
             cur["host_out"].copy_(cur["s_probs"], non_blocking=True)
+            if i in decode_checks:
+                hs = cur["host_status"][:cur["status"].numel()]
+                hs.copy_(cur["status"], non_blocking=True)
+                decode_checks[i] = (decode_checks[i], hs)
             cur["done"].record(main)
             self.last_logits = cur["s_logits"]
             if pending is not None:
-                pending["done"].synchronize()
-                yield pending["host_out"].clone()
+                yield finish(pending, i - 1)
             pending, i = cur, i + 1
-        pending["done"].synchronize()
-        yield pending["host_out"].clone()
+        yield finish(pending, i - 1)
 
     def compile(self, optimizer=None, loss=None, metrics=None, top_k: int = 5, **_):
         """Keras `model.compile` as eval.py:62-70 uses it: the loss and the two metrics are fixed

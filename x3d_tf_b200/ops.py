@@ -159,6 +159,36 @@ def video_clips_u8(frames: torch.Tensor, frame_off: torch.Tensor, desc: torch.Te
     return out
 
 
+def jpeg_entropy(data: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int,
+                 coef: torch.Tensor, status: torch.Tensor) -> None:
+    """x3d_jpeg_entropy: Huffman-decode `nframes` frames (`frames` / `tables`: the x3d_jpeg_frame /
+    x3d_jpeg_tables records as raw uint8 device buffers, validated on the host by video.pack_jpeg)
+    into `coef` (int16 blocks x 64) and their status words (int32)."""
+    for t, name in ((data, "data"), (frames, "frames"), (tables, "tables"), (coef, "coef"), (status, "status")):
+        _req(t, name)
+    if coef.dtype != torch.int16 or status.dtype != torch.int32:
+        raise TypeError("jpeg_entropy: coef int16, status int32")
+    _launch("x3d_jpeg_entropy", lambda: lib().x3d_jpeg_entropy(
+        data.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, coef.data_ptr(), status.data_ptr(), _stream()))
+
+
+def jpeg_idct(coef: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int, max_blocks: int,
+              method: int, planes: torch.Tensor) -> None:
+    """x3d_jpeg_idct: dequantise + 8x8 IDCT (method _lib.X3D_JPEG_ISLOW / X3D_JPEG_IFAST) into `planes`."""
+    for t, name in ((coef, "coef"), (frames, "frames"), (tables, "tables"), (planes, "planes")):
+        _req(t, name)
+    _launch("x3d_jpeg_idct", lambda: lib().x3d_jpeg_idct(
+        coef.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, max_blocks, method, planes.data_ptr(), _stream()))
+
+
+def jpeg_color(planes: torch.Tensor, frames: torch.Tensor, nframes: int, max_pixels: int, out: torch.Tensor) -> None:
+    """x3d_jpeg_color: chroma upsampling + YCbCr -> RGB into the packed frames `out` (uint8)."""
+    for t, name in ((planes, "planes"), (frames, "frames"), (out, "out")):
+        _req(t, name)
+    _launch("x3d_jpeg_color", lambda: lib().x3d_jpeg_color(
+        planes.data_ptr(), frames.data_ptr(), nframes, max_pixels, out.data_ptr(), _stream()))
+
+
 def stem_tc_u8_fwd(x: torch.Tensor, mean, std, wc: torch.Tensor, bias: torch.Tensor,
                    norm_value: float = 255.0) -> torch.Tensor:
     """Tensor-core stem with the uint8 input stage fused into its loader; bf16 activations out."""

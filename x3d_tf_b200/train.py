@@ -18,7 +18,11 @@ Out of scope here as in eval.py's driver: video decoding and augmentation (`data
 `[T, H, W, 3]` (or `[k, T, H, W, 3]`: k training clips of one video) with an integer label, or,
 with `--decoded_videos`, decoded videos `[F, H, W, 3]` uint8 of any size: then every global-batch
 slot draws one random clip of its video (temporal start, short-side scale jitter, crop, flip;
-`video.train_plan`) and the resize / crop / flip run on the device (x3d_video_clips_u8);
+`video.train_plan`) and the resize / crop / flip run on the device (x3d_video_clips_u8); or, with
+`--use_tfrecord` (the reference's flag), globs of the reference's GZIP TFRecord files: the file list
+is shuffled per epoch with the epoch seed (the same on every rank), rank r reads files r::world,
+records stream through a shuffle buffer of 16 x the per-rank batch (dataloader.py:158-159) and
+repeat as needed, and the sampled JPEG frames are decoded on the device (x3d_jpeg_*);
 `--synthetic N` trains on N seeded random clips per epoch instead.  W&B / TensorBoard callbacks are
 not reproduced; the per-epoch log line carries the same quantities Keras prints.
 """
@@ -95,6 +99,53 @@ def video_clip_batches(items: List[Tuple[str, int]], gbatch: int, steps: int, se
         yield vb, np.asarray([items[j][1] for j in mine], np.int32)
 
 
+def tfrecord_rank_files(files: List[str], seed: int, rank: int = 0, world: int = 1) -> List[str]:
+    """This rank's files of an epoch: the list shuffled with the epoch seed (identically on every
+    rank), then every world-th file from position `rank`."""
+    if len(files) < world:
+        raise ValueError(f"{len(files)} TFRecord files for {world} ranks: every rank needs at least one")
+    order = np.random.default_rng(seed).permutation(len(files))
+    return [files[i] for i in order[rank::world]]
+
+
+def tfrecord_clip_batches(files: List[str], gbatch: int, steps: int, seed: int, cfg, rank: int = 0,
+                          world: int = 1, crop_size: int = 0, dct_method: str = "INTEGER_FAST"):
+    """Exactly `steps` batches of this rank's share of the global batch as video.VideoBatch of JPEG
+    frames: the records of tfrecord_rank_files(...) in file order, repeated as needed, through a
+    shuffle buffer of 16 x the per-rank batch; one random clip per video, the clip draws from
+    video.train_rng(seed, rank).  The buffer holds whole parsed records (every JPEG frame of each
+    video, a few MB per 300-frame record), so its host memory grows with the batch: about 16 x batch
+    x the record size, as with tf.data's shuffle buffer in the reference."""
+    from . import tfrecord, video
+    batch = gbatch // world
+    mine = tfrecord_rank_files(files, seed, rank, world)
+    rng = video.train_rng(seed, rank)
+    pick = np.random.default_rng((int(seed), int(rank), 1))           # the shuffle buffer's draws
+
+    def records():
+        while True:
+            n = 0
+            for path in mine:
+                for v in tfrecord.read_videos(path):
+                    n += 1
+                    yield v
+            if n == 0:
+                raise ValueError(f"rank {rank}: its TFRecord files hold no records")
+
+    src, pool = records(), []
+    for _ in range(steps):
+        chosen = []
+        while len(chosen) < batch:
+            while len(pool) < 16 * batch:
+                pool.append(next(src))
+            j = int(pick.integers(0, len(pool)))
+            chosen.append(pool[j])
+            pool[j] = pool[-1]
+            pool.pop()
+        yield (video.train_batch(chosen, cfg, rng, crop_size, dct_method),
+               np.asarray([v.label for v in chosen], np.int32))
+
+
 def synthetic_clip_batches(steps: int, batch: int, T: int, S: int, num_classes: int, seed: int
                            ) -> Iterator[Tuple[np.ndarray, np.ndarray]]:
     rng = np.random.default_rng(seed)
@@ -110,6 +161,10 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     ap.add_argument("--val_file_pattern", default=None)
     ap.add_argument("--decoded_videos", action="store_true",
                     help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
+    ap.add_argument("--use_tfrecord", action="store_true",
+                    help="the file patterns are globs of GZIP TFRecord files (JPEG frames, decoded on the device)")
+    ap.add_argument("--dct_method", default="INTEGER_FAST", choices=["INTEGER_FAST", "INTEGER_ACCURATE"],
+                    help="IDCT of the JPEG decoder (tf.io.decode_jpeg's names; INTEGER_FAST is its default)")
     ap.add_argument("--model_dir", required=True)
     ap.add_argument("--pretrained_ckpt", default=None)
     ap.add_argument("--num_gpus", type=int, default=1)
@@ -124,6 +179,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     a = ap.parse_args(argv)
     if not a.train_file_pattern and not a.synthetic:
         ap.error("one of --train_file_pattern / --synthetic is required")
+    if a.use_tfrecord and a.decoded_videos:
+        ap.error("--use_tfrecord and --decoded_videos are mutually exclusive")
     if a.config.endswith(".yaml"):
         cfg = get_default_config(); cfg.merge_from_file(a.config); cfg.freeze()
     else:
@@ -151,7 +208,7 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     from .arch import build_arch
     from .model import X3D, keras_default_weights, reset_block_counters
     from .training import X3DTrainer
-    from .eval import file_batches, video_batches
+    from .eval import file_batches, tfrecord_batches, tfrecord_files, video_batches
     from .video import VideoBatch
 
     tr = X3DTrainer(cfg, device=dev, world=world, rank=rank)
@@ -177,10 +234,11 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     epochs = a.epochs or cfg.TRAIN.EPOCHS
     steps = a.steps_per_epoch or max(cfg.TRAIN.DATASET_SIZE // gbatch, 1)
     T, S = cfg.DATA.TEMP_DURATION, a.crop_size or cfg.DATA.TRAIN_CROP_SIZE
-    items = read_file_list(a.train_file_pattern) if a.train_file_pattern else None
+    read_list = tfrecord_files if a.use_tfrecord else read_file_list
+    items = read_list(a.train_file_pattern) if a.train_file_pattern else None
     if a.synthetic:
         steps = min(steps, max(a.synthetic // gbatch, 1))
-    val_items = read_file_list(a.val_file_pattern) if a.val_file_pattern else None
+    val_items = read_list(a.val_file_pattern) if a.val_file_pattern else None
     mean, std = tuple(cfg.DATA.MEAN), tuple(cfg.DATA.STD)
     history = []
     for epoch in range(current_epoch, epochs):
@@ -188,7 +246,10 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
         if rank == 0:
             print(f"\nEpoch {epoch + 1}/{epochs}\nEpoch {epoch + 1:05d}: LearningRateScheduler setting learning rate to {lr}.")
         # every rank runs exactly `steps` steps (rank-independent count; short lists repeat)
-        if items is not None and a.decoded_videos:
+        if items is not None and a.use_tfrecord:
+            data = tfrecord_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size,
+                                         a.dct_method)
+        elif items is not None and a.decoded_videos:
             data = video_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size)
         else:
             data = (file_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, rank, world) if items is not None
@@ -219,8 +280,13 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
             from .shard import shard_range
             lo, hi = shard_range(len(val_items), world, rank)
             vpb = max(cfg.TEST.BATCH_SIZE // num_preds, 1)
-            res = m.evaluate(video_batches(val_items[lo:hi], vpb, cfg) if a.decoded_videos
-                             else file_batches(val_items[lo:hi], vpb, num_preds))
+            if a.use_tfrecord:
+                val = tfrecord_batches(val_items[lo:hi], vpb, cfg, a.dct_method)
+            elif a.decoded_videos:
+                val = video_batches(val_items[lo:hi], vpb, cfg)
+            else:
+                val = file_batches(val_items[lo:hi], vpb, num_preds)
+            res = m.evaluate(val)
             log.update(val_loss=res["loss"], val_acc=res["acc"], val_top_5_acc=res["top_5_acc"])
             del m
         if rank == 0:

@@ -23,6 +23,11 @@ The resize is TF 2.4's ResizeBilinear with half_pixel_centers (what `tf.image.re
 "bilinear")` runs) followed by the cast back to uint8; include/x3d_b200.h states the arithmetic.
 Parity of these rules with TensorFlow is unpinned (TensorFlow is not available to this project's
 tests); they are restated from the reference's source.
+
+Videos read from the reference's TFRecords (tfrecord.TFRecordVideo, JPEG frames) are packed by
+`pack_jpeg` instead of `pack`: the batch then carries the entropy-coded segments of the distinct
+frames and their headers' tables (EncodedFrames), and the frames are decoded on the device
+(x3d_jpeg_entropy / _idct / _color) into the packed buffer the clip kernel reads.
 """
 from __future__ import annotations
 
@@ -164,6 +169,73 @@ def validate(plan: ClipPlan, shapes: Sequence[Sequence[int]]) -> None:
             raise ValueError(f"clip {n}: frame index outside 0..{F - 1}")
 
 
+DCT_METHODS = {"INTEGER_FAST": 1, "INTEGER_ACCURATE": 0}          # X3D_JPEG_IFAST / X3D_JPEG_ISLOW
+STATUS_TEXT = {1: "invalid Huffman code", 2: "run of coefficients past coefficient 63",
+               3: "premature end of the entropy-coded data"}
+
+
+def _align16(n: int) -> int:
+    return (n + 15) & ~15
+
+
+@dataclass
+class EncodedFrames:
+    """The JPEG frames of a VideoBatch, on the host (pinned when a CUDA device is present):
+    `data` the entropy-coded segments of the distinct frames, `frames` / `tables` their
+    x3d_jpeg_frame / x3d_jpeg_tables records (raw bytes), the sizes of the device buffers the
+    three decode stages use, the IDCT (`method`, DCT_METHODS) and a name per frame for messages."""
+    data: torch.Tensor          # [bytes] uint8
+    frames: torch.Tensor        # [nframes * 64] uint8
+    tables: torch.Tensor        # [ntables * 4200] uint8
+    nframes: int
+    coef_blocks: int
+    plane_bytes: int
+    out_bytes: int
+    max_blocks: int
+    max_pixels: int
+    method: int
+    names: List[str]
+
+    @property
+    def h2d_bytes(self) -> int:
+        return self.data.numel() + self.frames.numel() + self.tables.numel()
+
+    def decode(self, device, scratch: dict) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Copy to `device` and decode on the current stream into buffers kept in `scratch` (grown
+        as needed, reused while large enough).  Returns (decoded frames uint8, status int32
+        [nframes]); the status words are only valid once the stream has reached them."""
+        from . import ops
+
+        def buf(name, n, dtype):
+            t = scratch.get(name)
+            if t is None or t.numel() < n:
+                t = scratch[name] = torch.empty(max(n, 1), dtype=dtype, device=device)
+            return t[:max(n, 1)]
+
+        data, frames, tables = (buf(f"jpeg_{k}", v.numel(), torch.uint8) for k, v in
+                                (("data", self.data), ("frames", self.frames), ("tables", self.tables)))
+        data.copy_(self.data, non_blocking=True)
+        frames.copy_(self.frames, non_blocking=True)
+        tables.copy_(self.tables, non_blocking=True)
+        coef = buf("jpeg_coef", self.coef_blocks * 64, torch.int16)
+        planes = buf("jpeg_planes", self.plane_bytes, torch.uint8)
+        out = buf("frames", self.out_bytes, torch.uint8)
+        status = buf("jpeg_status", self.nframes, torch.int32)
+        ops.jpeg_entropy(data, frames, tables, self.nframes, coef, status)
+        ops.jpeg_idct(coef, frames, tables, self.nframes, self.max_blocks, self.method, planes)
+        ops.jpeg_color(planes, frames, self.nframes, self.max_pixels, out)
+        return out, status
+
+    def check(self, status) -> None:
+        """Raises ValueError naming the record and frame of the first nonzero status word (TF's
+        decode_jpeg with try_recover_truncated=False fails on such a frame too)."""
+        st = np.asarray(status).reshape(-1)[:self.nframes]
+        bad = np.flatnonzero(st)
+        if bad.size:
+            i = int(bad[0])
+            raise ValueError(f"{self.names[i]}: JPEG decoding failed: {STATUS_TEXT.get(int(st[i]), int(st[i]))}")
+
+
 @dataclass
 class VideoBatch:
     """Everything one x3d_video_clips_u8 launch needs, on the host: the distinct frames the plan
@@ -174,16 +246,25 @@ class VideoBatch:
     frame_off: torch.Tensor     # [N*T] int64
     desc: torch.Tensor          # [N, 7] int32
     shape: Tuple[int, int, int, int, int]
+    encoded: Optional[EncodedFrames] = None   # JPEG frames (pack_jpeg): `frames` is empty, and
+                                              # frame_off points into the frames they decode to
 
     @property
     def h2d_bytes(self) -> int:
-        return self.frames.numel() + self.frame_off.numel() * 8 + self.desc.numel() * 4
+        enc = self.encoded.h2d_bytes if self.encoded is not None else 0
+        return self.frames.numel() + self.frame_off.numel() * 8 + self.desc.numel() * 4 + enc
 
     def clips(self, device=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Copy to `device` and build the clips there (current stream)."""
+        """Copy to `device` and build the clips there (current stream).  JPEG frames are decoded
+        first; their status words are checked before this returns (a synchronisation), so a
+        corrupt frame raises ValueError here."""
         from . import ops
         device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        frames = self.frames.to(device, non_blocking=True)
+        if self.encoded is not None:
+            frames, status = self.encoded.decode(device, {})
+            self.encoded.check(status.cpu().numpy())
+        else:
+            frames = self.frames.to(device, non_blocking=True)
         off = self.frame_off.to(device, non_blocking=True)
         desc = self.desc.to(device, non_blocking=True)
         return ops.video_clips_u8(frames, off, desc, self.shape[1], self.shape[2], out=out)
@@ -218,6 +299,74 @@ def pack(videos: Sequence[np.ndarray], plan: ClipPlan, pin: Optional[bool] = Non
     return VideoBatch(buf, off, desc, plan.shape)
 
 
+def pack_jpeg(videos: Sequence, plan: ClipPlan, pin: Optional[bool] = None,
+              dct_method: str = "INTEGER_FAST") -> VideoBatch:
+    """`pack` for videos of JPEG frames (tfrecord.TFRecordVideo, or anything with `shape` and
+    `jpeg(f)` -> bytes): the entropy-coded segment of each distinct (video, frame) pair the plan
+    reads, once, in one buffer; a table set per distinct header; the frame descriptors and the
+    offsets of the decoded frames (16-byte aligned) that frame_off points at.  Headers are parsed
+    and checked here (jpeg.parse), so an unsupported or mis-sized frame raises ValueError naming
+    its video and frame before anything reaches the device.  `dct_method`: TF's decode_jpeg
+    names, INTEGER_FAST (its default) or INTEGER_ACCURATE."""
+    from . import jpeg as J
+    if dct_method not in DCT_METHODS:
+        raise ValueError(f"dct_method {dct_method!r}: INTEGER_FAST or INTEGER_ACCURATE")
+    shapes = [tuple(int(x) for x in v.shape) for v in videos]
+    validate(plan, shapes)
+    N, T = plan.frames.shape
+    keys = plan.video[:, None] * (1 << 32) + plan.frames
+    uniq, inv = np.unique(keys.reshape(-1), return_inverse=True)
+    recs = np.zeros(len(uniq), J.FRAME_DTYPE)
+    table_index, table_recs, segs, names = {}, [], [], []
+    seg_off = coef = plane = out = 0
+    max_blocks = max_pixels = 0
+    for n, k in enumerate(uniq):
+        v, f = int(k >> 32), int(k & 0xffffffff)
+        name = f"{getattr(videos[v], 'name', f'video {v}')} frame {f}"
+        buf = videos[v].jpeg(f)
+        try:
+            fr = J.parse(buf)
+        except ValueError as e:
+            raise ValueError(f"{name}: {e}") from None
+        h = fr.header
+        if (h.H, h.W) != shapes[v][1:3]:
+            raise ValueError(f"{name}: {h.H}x{h.W}, but frame 0 of its video is {shapes[v][1]}x{shapes[v][2]}")
+        t = table_index.get(id(h))
+        if t is None:
+            t = table_index[id(h)] = len(table_recs)
+            table_recs.append(h)
+        mcux, mcuy = -(-h.W // (8 * h.hs)), -(-h.H // (8 * h.vs))
+        blocks = mcux * mcuy * (h.hs * h.vs + 2)
+        recs[n] = (seg_off, coef, plane, out, fr.seg_len, h.H, h.W, h.hs, h.vs, t, n, 0)
+        segs.append(memoryview(buf)[fr.seg_off:fr.seg_off + fr.seg_len])
+        names.append(name)
+        seg_off += fr.seg_len
+        coef += blocks
+        plane += blocks * 64
+        out += _align16(h.H * h.W * 3)
+        max_blocks, max_pixels = max(max_blocks, blocks), max(max_pixels, h.H * h.W)
+    if pin is None:
+        pin = torch.cuda.is_available()
+    data = torch.empty(max(seg_off, 1), dtype=torch.uint8, pin_memory=bool(pin))
+    host = data.numpy()
+    for r, sg in zip(recs, segs):
+        host[r["seg_off"]:r["seg_off"] + len(sg)] = np.frombuffer(sg, np.uint8)
+    tables = np.stack([h.tables for h in table_recs])
+    frames_t = torch.from_numpy(recs.view(np.uint8).copy())
+    tables_t = torch.from_numpy(tables.view(np.uint8).reshape(-1).copy())
+    off = torch.from_numpy(recs["out_off"][inv].reshape(N * T).astype(np.int64))
+    desc = torch.from_numpy(np.ascontiguousarray(plan.desc, np.int32))
+    if pin:
+        frames_t, tables_t, off, desc = (t.pin_memory() for t in (frames_t, tables_t, off, desc))
+    enc = EncodedFrames(data, frames_t, tables_t, len(uniq), coef, plane, out, max_blocks, max_pixels,
+                        DCT_METHODS[dct_method], names)
+    return VideoBatch(torch.empty(0, dtype=torch.uint8), off, desc, plan.shape, enc)
+
+
+def _pack(videos, plan: ClipPlan, dct_method: str) -> VideoBatch:
+    return pack_jpeg(videos, plan, dct_method=dct_method) if hasattr(videos[0], "jpeg") else pack(videos, plan)
+
+
 def load_video(path: str) -> np.ndarray:
     """A decoded video `.npy` [F, H, W, 3] uint8, memory-mapped (packing reads the sampled frames only)."""
     v = np.load(path, mmap_mode="r")
@@ -227,15 +376,16 @@ def load_video(path: str) -> np.ndarray:
     return v
 
 
-def eval_batch(videos: List[np.ndarray], cfg) -> VideoBatch:
-    """The evaluation clips of `videos` for cfg.DATA / cfg.TEST."""
+def eval_batch(videos: List[np.ndarray], cfg, dct_method: str = "INTEGER_FAST") -> VideoBatch:
+    """The evaluation clips of `videos` (decoded, or of JPEG frames) for cfg.DATA / cfg.TEST."""
     plan = eval_plan([v.shape for v in videos], cfg.DATA.TEMP_DURATION, cfg.TEST.NUM_TEMPORAL_VIEWS,
                      cfg.TEST.NUM_SPATIAL_CROPS, cfg.DATA.TEST_CROP_SIZE)
-    return pack(videos, plan)
+    return _pack(videos, plan, dct_method)
 
 
-def train_batch(videos: List[np.ndarray], cfg, rng: np.random.Generator, crop_size: int = 0) -> VideoBatch:
-    """One random training clip per video for cfg.DATA."""
+def train_batch(videos: List[np.ndarray], cfg, rng: np.random.Generator, crop_size: int = 0,
+                dct_method: str = "INTEGER_FAST") -> VideoBatch:
+    """One random training clip per video (decoded, or of JPEG frames) for cfg.DATA."""
     plan = train_plan([v.shape for v in videos], cfg.DATA.TEMP_DURATION, cfg.DATA.FRAME_RATE,
                       cfg.DATA.TRAIN_JITTER_SCALES, crop_size or cfg.DATA.TRAIN_CROP_SIZE, rng)
-    return pack(videos, plan)
+    return _pack(videos, plan, dct_method)
