@@ -347,6 +347,83 @@ int x3d_jpeg_idct(const int16_t* coef, const x3d_jpeg_frame* frames, const x3d_j
  * max_pixels >= H*W of every frame. */
 int x3d_jpeg_color(const uint8_t* planes, const x3d_jpeg_frame* frames, int nframes, int64_t max_pixels,
                    uint8_t* out, void* stream);
+/* ---- Baseline JPEG encoding of video frames --------------------------------------------------------
+ * Replaces the reference's tf.io.encode_jpeg(frame, quality=90) of every frame
+ * (datasets/create_tfrecords.py:48-83).  These four stages reproduce libjpeg-turbo's compressor with
+ * TF's settings bit for bit: JDCT_ISLOW, jpeg_set_quality(q, force_baseline = TRUE), the standard
+ * (Annex K) Huffman tables or any others given in x3d_jpeg_enc_tables, no restart interval, three
+ * components, luma sampling 2x2 (4:2:0) or 1x1 (4:4:4).  Each stage covers a ragged batch in one call
+ * (one launch; two for the stuffing stage).
+ * The host writes the headers (x3d_tf_b200/jpeg.py encoder_header) and appends EOI.
+ *
+ * Input: packed row-major [H][W][3] RGB uint8 frames at in_off in `rgb` (the layout x3d_jpeg_color
+ * writes and x3d_video_clips_u8 reads).  Coefficients use the decoder's layout (above): component
+ * after component, mcux*hs x mcuy*vs luma blocks then mcux x mcuy blocks of Cb and of Cr, int16 natural
+ * order, block b at coef + (coef_off + b) * 64.  A frame's bit stream is MSB first in 32-bit words at
+ * word_off in `words` (bit 0 = bit 31 of the first word); its entropy-coded segment (byte stuffing
+ * included, padded with 1-bits) lands in `out` at the result's out_off.
+ * The descriptors are device data and are NOT checked by the calls; the caller guarantees per frame:
+ * 1 <= H, W <= 65535; hs = vs in {1, 2}; 0 <= tables < the number of table sets; the input frame, the
+ * coefficient blocks, boff[coef_off .. + blocks) and words[word_off .. + word_cap) inside their
+ * buffers; ranges of different frames do not overlap.  word_cap >= blocks * 52 + 1 always suffices
+ * (a block codes to at most 1660 bits); a frame that needs more gets X3D_JPEG_OVERFLOW. */
+typedef struct x3d_jpeg_enc_frame {
+  int64_t in_off;      /* first byte of the RGB frame */
+  int64_t coef_off;    /* first coefficient block, and first entry of boff */
+  int64_t word_off;    /* first 32-bit word of the bit stream */
+  int64_t word_cap;    /* words available there */
+  int32_t H, W;
+  int32_t hs, vs;      /* luma sampling factors: (2, 2) or (1, 1) */
+  int32_t tables;      /* index of its x3d_jpeg_enc_tables */
+  int32_t reserved;
+} x3d_jpeg_enc_frame;
+/* Quantisation tables (natural order: luma, chroma) and Huffman codes by symbol (jchuff.c
+ * jpeg_make_c_derived_tbl ehufco / ehufsi) of DC luma, AC luma, DC chroma, AC chroma. */
+typedef struct x3d_jpeg_enc_tables {
+  uint16_t q[2][64];
+  uint16_t code[4][256];
+  uint8_t size[4][256];
+} x3d_jpeg_enc_tables;
+/* Per frame: bits of the entropy-coded data before padding (x3d_jpeg_enc_bits), the start of its
+ * region in `out` (x3d_jpeg_enc_stuff, every frame), the length of its segment with byte stuffing, and
+ * X3D_JPEG_OK or X3D_JPEG_OVERFLOW (word_cap or out_cap too small: then len is not written and
+ * nothing of the frame is written to `words` or `out`). */
+typedef struct x3d_jpeg_enc_result {
+  int64_t bits;
+  int64_t out_off;
+  int64_t len;
+  int32_t status;
+  int32_t reserved;
+} x3d_jpeg_enc_result;
+#define X3D_JPEG_OVERFLOW 4
+/* Stage A: jccolor.c rgb_ycc_convert (16-bit fixed point), the last column and row replicated
+ * (jcsample.c expand_right_edge, jcprepct.c expand_bottom_edge), chroma of 4:2:0 by jcsample.c
+ * h2v2_downsample (bias 1, 2) with its last row replicated to the MCU height, jfdctint.c
+ * jpeg_fdct_islow and jcdctmgr.c's quantisation by reciprocal (compute_reciprocal of q << 3 with
+ * libjpeg-turbo's 16-bit DCTELEM).  The luma blocks of 4:2:0 frames past ceil(W/8) x ceil(H/8) are
+ * jccoefct.c's dummy blocks: AC zero, DC that of the block before them in the MCU.
+ * max_blocks >= the block count of every frame. */
+int x3d_jpeg_fdct(const uint8_t* rgb, const x3d_jpeg_enc_frame* frames, const x3d_jpeg_enc_tables* tables,
+                  int nframes, int max_blocks, int16_t* coef, void* stream);
+/* Stage B: the code length of every block (jchuff.c encode_one_block: DC difference to the previous
+ * block of the component in scan order, AC run lengths with ZRL and EOB), an exclusive scan per frame
+ * into boff[coef_off + scan position] (int64 bit offsets), res[f].bits and res[f].status, and zeroes
+ * the frame's ceil(bits / 32) words.  One CTA per frame. */
+int x3d_jpeg_enc_bits(const int16_t* coef, const x3d_jpeg_enc_frame* frames, const x3d_jpeg_enc_tables* tables,
+                      int nframes, int64_t* boff, x3d_jpeg_enc_result* res, uint32_t* words, void* stream);
+/* Stage C1: every block's codes ORed into the frame's words at its bit offset; the last block pads the
+ * stream to a byte with 1-bits (jchuff.c flush_bits).  Frames whose status is not X3D_JPEG_OK are
+ * skipped.  max_blocks as for x3d_jpeg_fdct. */
+int x3d_jpeg_enc_emit(const int16_t* coef, const x3d_jpeg_enc_frame* frames, const x3d_jpeg_enc_tables* tables,
+                      int nframes, int max_blocks, const int64_t* boff, const x3d_jpeg_enc_result* res,
+                      uint32_t* words, void* stream);
+/* Stage C2: byte stuffing (0x00 after every 0xFF) into `out` (out_cap bytes).  A first launch (one CTA)
+ * writes res[f].out_off for every frame: the sum over frames f' < f of 2 * ceil(bits_f' / 8), a bound
+ * of their stuffed lengths, so out_cap >= 2 * the sum over all frames suffices.  The second (one CTA per
+ * frame) stuffs every X3D_JPEG_OK frame whose region fits and writes res[f].len; a frame whose region
+ * ends past out_cap gets X3D_JPEG_OVERFLOW. */
+int x3d_jpeg_enc_stuff(const uint32_t* words, const x3d_jpeg_enc_frame* frames, int nframes,
+                       x3d_jpeg_enc_result* res, uint8_t* out, int64_t out_cap, void* stream);
 
 /* x3d_stem_tc_fwd with the input stage fused into its loader: uint8 NDHWC clips in, bf16
  * activations out (same result as x3d_normalize_u8(bf16) followed by x3d_stem_tc_fwd). */

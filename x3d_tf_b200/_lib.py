@@ -63,7 +63,23 @@ class JpegTables(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class JpegEncFrame(C.Structure):
+    _fields_ = [("in_off", C.c_int64), ("coef_off", C.c_int64), ("word_off", C.c_int64), ("word_cap", C.c_int64),
+                ("H", C.c_int32), ("W", C.c_int32), ("hs", C.c_int32), ("vs", C.c_int32), ("tables", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
+class JpegEncTables(C.Structure):
+    _fields_ = [("q", (C.c_uint16 * 64) * 2), ("code", (C.c_uint16 * 256) * 4), ("size", (C.c_uint8 * 256) * 4)]
+
+
+class JpegEncResult(C.Structure):
+    _fields_ = [("bits", C.c_int64), ("out_off", C.c_int64), ("len", C.c_int64), ("status", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 X3D_JPEG_ISLOW, X3D_JPEG_IFAST = 0, 1
+X3D_JPEG_OVERFLOW = 4
 
 # name -> (restype, argtypes); must list every symbol include/x3d_b200.h declares.
 SIGNATURES = {
@@ -133,6 +149,10 @@ SIGNATURES = {
     "x3d_jpeg_entropy": (C.c_int, [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3),
     "x3d_jpeg_idct": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p] * 2),
     "x3d_jpeg_color": (C.c_int, [C.c_void_p] * 2 + [C.c_int, C.c_int64] + [C.c_void_p] * 2),
+    "x3d_jpeg_fdct": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 2 + [C.c_void_p] * 2),
+    "x3d_jpeg_enc_bits": (C.c_int, [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 4),
+    "x3d_jpeg_enc_emit": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 2 + [C.c_void_p] * 4),
+    "x3d_jpeg_enc_stuff": (C.c_int, [C.c_void_p] * 2 + [C.c_int] + [C.c_void_p] * 2 + [C.c_int64, C.c_void_p]),
     "x3d_stem_tc_u8_fwd": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_float,
                                      C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p]),
     "x3d_eval_metrics": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,

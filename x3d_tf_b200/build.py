@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libx3d_b200.so")
-SOURCES = ["host_util.cu", "x3d_simt.cu", "x3d_pw_tc.cu", "x3d_pw_tf32_tc.cu", "x3d_dw_tma.cu", "x3d_dw_planar.cu", "x3d_stem_tc.cu", "x3d_ab_fused.cu", "x3d_ab_persist.cu", "x3d_train.cu", "x3d_io.cu", "x3d_jpeg.cu"]
+SOURCES = ["host_util.cu", "x3d_simt.cu", "x3d_pw_tc.cu", "x3d_pw_tf32_tc.cu", "x3d_dw_tma.cu", "x3d_dw_planar.cu", "x3d_stem_tc.cu", "x3d_ab_fused.cu", "x3d_ab_persist.cu", "x3d_train.cu", "x3d_io.cu", "x3d_jpeg.cu", "x3d_jpeg_enc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default",
               "--expt-relaxed-constexpr"]

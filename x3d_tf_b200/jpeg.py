@@ -294,3 +294,252 @@ def parse(buf) -> JpegFrame:
     if marker != 0xD9:
         raise ValueError(f"marker 0x{marker:02X} after the scan: only one scan followed by EOI is supported")
     return JpegFrame(h, h.scan_off, int(ff[0]))
+
+
+# ---- Encoder side: the tables and headers libjpeg-turbo's compressor writes with tf.io.encode_jpeg's
+# settings (the reference's datasets/create_tfrecords.py:48-83): baseline, JDCT_ISLOW, standard
+# Huffman tables, jpeg_set_quality(q, force_baseline=TRUE), no restart interval, JFIF 1.01 APP0 with
+# 300x300 dpi.  The entropy-coded segments come from the device (x3d_jpeg_fdct / _enc_bits / _emit /
+# _stuff, include/x3d_b200.h).
+
+# jcparam.c std_luminance_quant_tbl / std_chrominance_quant_tbl (ITU T.81 Annex K.1), natural order
+STD_QUANT = np.array([
+    [16, 11, 10, 16, 24, 40, 51, 61, 12, 12, 14, 19, 26, 58, 60, 55, 14, 13, 16, 24, 40, 57, 69, 56,
+     14, 17, 22, 29, 51, 87, 80, 62, 18, 22, 37, 56, 68, 109, 103, 77, 24, 35, 55, 64, 81, 104, 113, 92,
+     49, 64, 78, 87, 103, 121, 120, 101, 72, 92, 95, 98, 112, 100, 103, 99],
+    [17, 18, 24, 47] + [99] * 4 + [18, 21, 26, 66] + [99] * 4 + [24, 26, 56] + [99] * 5 + [47, 66] + [99] * 38],
+    np.int64)
+
+# jcparam.c std_huff_tables (Annex K.3): (bits[1..16], huffval) of DC luma, AC luma, DC chroma, AC chroma
+STD_HUFF = (
+    ([0, 1, 5, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0, 0, 0], list(range(12))),
+    ([0, 2, 1, 3, 3, 2, 4, 3, 5, 5, 4, 4, 0, 0, 1, 0x7D], [
+        0x01, 0x02, 0x03, 0x00, 0x04, 0x11, 0x05, 0x12, 0x21, 0x31, 0x41, 0x06, 0x13, 0x51, 0x61, 0x07,
+        0x22, 0x71, 0x14, 0x32, 0x81, 0x91, 0xA1, 0x08, 0x23, 0x42, 0xB1, 0xC1, 0x15, 0x52, 0xD1, 0xF0,
+        0x24, 0x33, 0x62, 0x72, 0x82, 0x09, 0x0A, 0x16, 0x17, 0x18, 0x19, 0x1A, 0x25, 0x26, 0x27, 0x28,
+        0x29, 0x2A, 0x34, 0x35, 0x36, 0x37, 0x38, 0x39, 0x3A, 0x43, 0x44, 0x45, 0x46, 0x47, 0x48, 0x49,
+        0x4A, 0x53, 0x54, 0x55, 0x56, 0x57, 0x58, 0x59, 0x5A, 0x63, 0x64, 0x65, 0x66, 0x67, 0x68, 0x69,
+        0x6A, 0x73, 0x74, 0x75, 0x76, 0x77, 0x78, 0x79, 0x7A, 0x83, 0x84, 0x85, 0x86, 0x87, 0x88, 0x89,
+        0x8A, 0x92, 0x93, 0x94, 0x95, 0x96, 0x97, 0x98, 0x99, 0x9A, 0xA2, 0xA3, 0xA4, 0xA5, 0xA6, 0xA7,
+        0xA8, 0xA9, 0xAA, 0xB2, 0xB3, 0xB4, 0xB5, 0xB6, 0xB7, 0xB8, 0xB9, 0xBA, 0xC2, 0xC3, 0xC4, 0xC5,
+        0xC6, 0xC7, 0xC8, 0xC9, 0xCA, 0xD2, 0xD3, 0xD4, 0xD5, 0xD6, 0xD7, 0xD8, 0xD9, 0xDA, 0xE1, 0xE2,
+        0xE3, 0xE4, 0xE5, 0xE6, 0xE7, 0xE8, 0xE9, 0xEA, 0xF1, 0xF2, 0xF3, 0xF4, 0xF5, 0xF6, 0xF7, 0xF8,
+        0xF9, 0xFA]),
+    ([0, 3, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0], list(range(12))),
+    ([0, 2, 1, 2, 4, 4, 3, 4, 7, 5, 4, 4, 0, 1, 2, 0x77], [
+        0x00, 0x01, 0x02, 0x03, 0x11, 0x04, 0x05, 0x21, 0x31, 0x06, 0x12, 0x41, 0x51, 0x07, 0x61, 0x71,
+        0x13, 0x22, 0x32, 0x81, 0x08, 0x14, 0x42, 0x91, 0xA1, 0xB1, 0xC1, 0x09, 0x23, 0x33, 0x52, 0xF0,
+        0x15, 0x62, 0x72, 0xD1, 0x0A, 0x16, 0x24, 0x34, 0xE1, 0x25, 0xF1, 0x17, 0x18, 0x19, 0x1A, 0x26,
+        0x27, 0x28, 0x29, 0x2A, 0x35, 0x36, 0x37, 0x38, 0x39, 0x3A, 0x43, 0x44, 0x45, 0x46, 0x47, 0x48,
+        0x49, 0x4A, 0x53, 0x54, 0x55, 0x56, 0x57, 0x58, 0x59, 0x5A, 0x63, 0x64, 0x65, 0x66, 0x67, 0x68,
+        0x69, 0x6A, 0x73, 0x74, 0x75, 0x76, 0x77, 0x78, 0x79, 0x7A, 0x82, 0x83, 0x84, 0x85, 0x86, 0x87,
+        0x88, 0x89, 0x8A, 0x92, 0x93, 0x94, 0x95, 0x96, 0x97, 0x98, 0x99, 0x9A, 0xA2, 0xA3, 0xA4, 0xA5,
+        0xA6, 0xA7, 0xA8, 0xA9, 0xAA, 0xB2, 0xB3, 0xB4, 0xB5, 0xB6, 0xB7, 0xB8, 0xB9, 0xBA, 0xC2, 0xC3,
+        0xC4, 0xC5, 0xC6, 0xC7, 0xC8, 0xC9, 0xCA, 0xD2, 0xD3, 0xD4, 0xD5, 0xD6, 0xD7, 0xD8, 0xD9, 0xDA,
+        0xE2, 0xE3, 0xE4, 0xE5, 0xE6, 0xE7, 0xE8, 0xE9, 0xEA, 0xF2, 0xF3, 0xF4, 0xF5, 0xF6, 0xF7, 0xF8,
+        0xF9, 0xFA]),
+)
+
+CHROMA = {"420": (2, 2), "444": (1, 1)}                 # encode_jpeg chroma_downsampling True / False
+ENC_FRAME_DTYPE = np.dtype(_lib.JpegEncFrame)
+ENC_RESULT_DTYPE = np.dtype(_lib.JpegEncResult)
+EOI = b"\xff\xd9"
+
+
+def quant_tables(quality: int) -> np.ndarray:
+    """[2, 64] uint16 luma / chroma quantisation tables, natural order: jcparam.c jpeg_set_quality
+    (jpeg_quality_scaling, then jpeg_add_quant_table with force_baseline = TRUE)."""
+    q = min(max(int(quality), 1), 100)
+    scale = 5000 // q if q < 50 else 200 - 2 * q
+    t = (STD_QUANT * scale + 50) // 100
+    return np.clip(t, 1, 255).astype(np.uint16)
+
+
+def huff_codes(bits, huffval):
+    """jchuff.c jpeg_make_c_derived_tbl: (ehufco[256], ehufsi[256]) code and length by symbol."""
+    co, si = np.zeros(256, np.uint32), np.zeros(256, np.uint8)
+    code, p = 0, 0
+    for l in range(1, 17):
+        for _ in range(bits[l - 1]):
+            co[huffval[p]], si[huffval[p]] = code, l
+            code += 1
+            p += 1
+        code <<= 1
+    return co, si
+
+
+def _segment(marker: int, body: bytes) -> bytes:
+    return bytes([0xFF, marker]) + (len(body) + 2).to_bytes(2, "big") + body
+
+
+def encoder_header(H: int, W: int, quality: int = 90, subsampling: str = "420") -> bytes:
+    """Everything before the entropy-coded segment, as libjpeg-turbo writes it (jcmarker.c): SOI,
+    JFIF 1.01 APP0 with 300x300 dpi, DQT luma, DQT chroma (zigzag order), SOF0, DHT DC0, AC0, DC1,
+    AC1, SOS of the three components."""
+    if subsampling not in CHROMA:
+        raise ValueError(f"subsampling {subsampling!r}: '420' or '444'")
+    if not (1 <= H <= 65535 and 1 <= W <= 65535):
+        raise ValueError(f"frame size {H}x{W}: 1..65535 each")
+    hs, vs = CHROMA[subsampling]
+    qt = quant_tables(quality)
+    out = b"\xff\xd8" + _segment(0xE0, b"JFIF\0\x01\x01\x01" + (300).to_bytes(2, "big") * 2 + b"\0\0")
+    for i in range(2):
+        out += _segment(0xDB, bytes([i]) + bytes(qt[i][ZIGZAG].astype(np.uint8)))
+    out += _segment(0xC0, bytes([8]) + H.to_bytes(2, "big") + W.to_bytes(2, "big") +
+                    bytes([3, 1, hs << 4 | vs, 0, 2, 0x11, 1, 3, 0x11, 1]))
+    for cls_id, (bits, vals) in zip((0x00, 0x10, 0x01, 0x11), STD_HUFF):
+        out += _segment(0xC4, bytes([cls_id] + bits + vals))
+    return out + _segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))
+
+
+ENC_TABLES_DTYPE = np.dtype(_lib.JpegEncTables)
+WORDS_PER_BLOCK = 52            # a block codes to at most 11 + 11 + 63 * (16 + 10) = 1660 bits
+# blocks per launch group, which bounds the device scratch: per block 128 B of coefficients, 8 B of bit
+# offset, 52 words of bits (208 B) and 416 B of output bound, 760 B in all: 3.2 GB at 2^22 blocks (a
+# 600-frame 360x480 4:2:0 batch is 2.4 M blocks), plus the frames themselves
+MAX_LAUNCH_BLOCKS = 1 << 22
+
+_enc_tables: Dict[int, np.ndarray] = {}
+_headers: Dict[Tuple[int, int, int, str], bytes] = {}
+
+
+def enc_tables(quality: int) -> np.ndarray:
+    """The x3d_jpeg_enc_tables record of `quality`: quant_tables and the standard Huffman codes."""
+    t = _enc_tables.get(quality)
+    if t is None:
+        t = np.zeros((), ENC_TABLES_DTYPE)
+        t["q"] = quant_tables(quality)
+        for i, (bits, vals) in enumerate(STD_HUFF):
+            t["code"][i], t["size"][i] = huff_codes(bits, vals)
+        _enc_tables[quality] = t
+    return t
+
+
+def enc_blocks(H: int, W: int, hs: int) -> int:
+    """Coefficient blocks of an H x W frame with luma sampling hs x hs (dummy blocks included)."""
+    mcux, mcuy = -(-W // (8 * hs)), -(-H // (8 * hs))
+    return mcux * mcuy * (hs * hs + 2)
+
+
+def _as_frames(frames):
+    """A list of [H, W, 3] uint8 frames: torch tensors (on the device or the host) or numpy arrays
+    (memory-mapped ones are read once, into the pinned staging buffer)."""
+    import torch
+    if isinstance(frames, (list, tuple)):
+        items = list(frames)
+    else:
+        if frames.ndim == 3:
+            frames = frames[None]
+        if frames.ndim != 4:
+            raise ValueError(f"frames must be [F, H, W, 3] or [H, W, 3], got {tuple(frames.shape)}")
+        items = list(frames)
+    for i, f in enumerate(items):
+        dtype_ok = f.dtype == (torch.uint8 if isinstance(f, torch.Tensor) else np.uint8)
+        if not dtype_ok or f.ndim != 3 or f.shape[2] != 3:
+            raise ValueError(f"frame {i}: need uint8 [H, W, 3], got {f.dtype} {tuple(f.shape)}")
+        if not (1 <= f.shape[0] <= 65535 and 1 <= f.shape[1] <= 65535):
+            raise ValueError(f"frame {i}: size {f.shape[0]}x{f.shape[1]} (1..65535 each)")
+    return items
+
+
+def _on_device(f) -> bool:
+    return getattr(f, "is_cuda", False)
+
+
+def encode_frames(frames, quality: int = 90, chroma: str = "420", scratch: dict = None) -> list:
+    """Complete JPEG files of uint8 RGB frames, encoded on the current CUDA device exactly as
+    tf.io.encode_jpeg(frame, quality, chroma_downsampling=chroma == "420") (libjpeg-turbo) writes
+    them.  `frames`: [F, H, W, 3] or a ragged list of [H, W, 3], on the device or on the host
+    (pinned host memory is copied asynchronously).  `scratch` keeps the device buffers between
+    calls (grown as needed); after the call it also holds the last launch group's buffers."""
+    import torch
+    if chroma not in CHROMA:
+        raise ValueError(f"chroma {chroma!r}: '420' or '444'")
+    if not 1 <= int(quality) <= 100:
+        raise ValueError(f"quality {quality}: 1..100")
+    quality = int(quality)
+    hs = CHROMA[chroma][0]
+    items = _as_frames(frames)
+    scratch = {} if scratch is None else scratch
+    device = torch.device("cuda", torch.cuda.current_device())
+    out: list = []
+    i = 0
+    while i < len(items):
+        j, blocks = i, 0
+        while j < len(items) and (j == i or blocks + enc_blocks(*items[j].shape[:2], hs) <= MAX_LAUNCH_BLOCKS):
+            blocks += enc_blocks(*items[j].shape[:2], hs)
+            j += 1
+        out += _encode_group(items[i:j], quality, chroma, hs, scratch, device)
+        i = j
+    return out
+
+
+def _encode_group(items, quality, chroma, hs, scratch, device) -> list:
+    import torch
+    from . import ops
+
+    def buf(name, n, dtype, pin=False):
+        t = scratch.get(name)
+        if t is None or t.numel() < n:
+            t = scratch[name] = (torch.empty(max(n, 1), dtype=dtype, pin_memory=True) if pin else
+                                 torch.empty(max(n, 1), dtype=dtype, device=device))
+        return t[:max(n, 1)]
+
+    n = len(items)
+    recs = np.zeros(n, ENC_FRAME_DTYPE)
+    in_off = coef = word = 0
+    max_blocks = 0
+    for k, f in enumerate(items):
+        H, W = int(f.shape[0]), int(f.shape[1])
+        nb = enc_blocks(H, W, hs)
+        cap = nb * WORDS_PER_BLOCK + 1
+        recs[k] = (in_off, coef, word, cap, H, W, hs, hs, 0, 0)
+        in_off += H * W * 3
+        coef += nb
+        word += cap
+        max_blocks = max(max_blocks, nb)
+    # the frames, packed on the device (host frames through the pinned staging buffer)
+    if all(_on_device(f) for f in items):
+        rgb = torch.cat([f.reshape(-1) for f in items]) if len(items) > 1 else items[0].reshape(-1).contiguous()
+    else:
+        stage = buf("enc_rgb_host", in_off, torch.uint8, pin=True)
+        host = stage.numpy()
+        for k, f in enumerate(items):
+            o, size = int(recs[k]["in_off"]), int(np.prod(f.shape))
+            if isinstance(f, torch.Tensor):
+                stage[o:o + size].copy_(f.reshape(-1))
+            else:
+                host[o:o + size] = np.asarray(f).reshape(-1)
+        rgb = buf("enc_rgb", in_off, torch.uint8)
+        rgb.copy_(stage, non_blocking=True)
+    frames_t = torch.from_numpy(recs.view(np.uint8).copy()).to(device, non_blocking=False)
+    tables_t = torch.from_numpy(enc_tables(quality).reshape(1).view(np.uint8).copy()).to(device)
+    coef_t = buf("enc_coef", coef * 64, torch.int16)
+    boff = buf("enc_boff", coef, torch.int64)
+    res = buf("enc_res", n * ENC_RESULT_DTYPE.itemsize, torch.uint8)
+    words = buf("enc_words", word, torch.int32)
+    seg = buf("enc_out", word * 8, torch.uint8)
+    ops.jpeg_fdct(rgb, frames_t, tables_t, n, max_blocks, coef_t)
+    ops.jpeg_enc_bits(coef_t, frames_t, tables_t, n, boff, res, words)
+    ops.jpeg_enc_emit(coef_t, frames_t, tables_t, n, max_blocks, boff, res, words)
+    ops.jpeg_enc_stuff(words, frames_t, n, res, seg)
+    scratch.update(enc_frames=frames_t, enc_coef_group=coef_t, enc_res_group=res, enc_out_group=seg)
+    r = res.cpu().numpy().view(ENC_RESULT_DTYPE)            # synchronises
+    bad = np.flatnonzero(r["status"] != 0)
+    if bad.size:
+        raise RuntimeError(f"JPEG encoding of frame {int(bad[0])} failed with status {int(r['status'][bad[0]])}")
+    end = int((r["out_off"] + r["len"]).max())
+    out_host = buf("enc_out_host", end, torch.uint8, pin=True)
+    out_host.copy_(seg[:end])
+    mv = memoryview(out_host.numpy())
+    files = []
+    for k, f in enumerate(items):
+        key = (int(f.shape[0]), int(f.shape[1]), quality, chroma)
+        hdr = _headers.get(key)
+        if hdr is None:
+            if len(_headers) > 4096:
+                _headers.clear()
+            hdr = _headers[key] = encoder_header(*key)
+        o = int(r["out_off"][k])
+        files.append(b"".join((hdr, mv[o:o + int(r["len"][k])], EOI)))
+    return files

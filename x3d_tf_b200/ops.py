@@ -189,6 +189,56 @@ def jpeg_color(planes: torch.Tensor, frames: torch.Tensor, nframes: int, max_pix
         planes.data_ptr(), frames.data_ptr(), nframes, max_pixels, out.data_ptr(), _stream()))
 
 
+def _req_all(what: str, dtypes: dict) -> None:
+    for name, (t, dtype) in dtypes.items():
+        _req(t, name)
+        if t.dtype != dtype:
+            raise TypeError(f"{what}: {name} must be {dtype}, got {t.dtype}")
+
+
+def jpeg_fdct(rgb: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int, max_blocks: int,
+              coef: torch.Tensor) -> None:
+    """x3d_jpeg_fdct: colour conversion, downsampling, ISLOW FDCT and quantisation of `nframes` packed RGB
+    frames (`frames` / `tables`: x3d_jpeg_enc_frame / x3d_jpeg_enc_tables records as raw uint8 device
+    buffers, built by jpeg.encode_frames) into `coef` (int16 blocks x 64)."""
+    _req_all("jpeg_fdct", {"rgb": (rgb, torch.uint8), "frames": (frames, torch.uint8),
+                           "tables": (tables, torch.uint8), "coef": (coef, torch.int16)})
+    _launch("x3d_jpeg_fdct", lambda: lib().x3d_jpeg_fdct(
+        rgb.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, max_blocks, coef.data_ptr(), _stream()))
+
+
+def jpeg_enc_bits(coef: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int, boff: torch.Tensor,
+                  res: torch.Tensor, words: torch.Tensor) -> None:
+    """x3d_jpeg_enc_bits: the bit offset of every block (int64 `boff`), each frame's bit count and status
+    (x3d_jpeg_enc_result records in the uint8 `res`), and the frame's words zeroed."""
+    _req_all("jpeg_enc_bits", {"coef": (coef, torch.int16), "frames": (frames, torch.uint8),
+                               "tables": (tables, torch.uint8), "boff": (boff, torch.int64),
+                               "res": (res, torch.uint8), "words": (words, torch.int32)})
+    _launch("x3d_jpeg_enc_bits", lambda: lib().x3d_jpeg_enc_bits(
+        coef.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, boff.data_ptr(), res.data_ptr(),
+        words.data_ptr(), _stream()))
+
+
+def jpeg_enc_emit(coef: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int, max_blocks: int,
+                  boff: torch.Tensor, res: torch.Tensor, words: torch.Tensor) -> None:
+    """x3d_jpeg_enc_emit: every block's Huffman codes into the frame's 32-bit words (int32 `words`)."""
+    _req_all("jpeg_enc_emit", {"coef": (coef, torch.int16), "frames": (frames, torch.uint8),
+                               "tables": (tables, torch.uint8), "boff": (boff, torch.int64),
+                               "res": (res, torch.uint8), "words": (words, torch.int32)})
+    _launch("x3d_jpeg_enc_emit", lambda: lib().x3d_jpeg_enc_emit(
+        coef.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, max_blocks, boff.data_ptr(), res.data_ptr(),
+        words.data_ptr(), _stream()))
+
+
+def jpeg_enc_stuff(words: torch.Tensor, frames: torch.Tensor, nframes: int, res: torch.Tensor,
+                   out: torch.Tensor) -> None:
+    """x3d_jpeg_enc_stuff: byte stuffing into `out` (uint8); each segment's offset and length in `res`."""
+    _req_all("jpeg_enc_stuff", {"words": (words, torch.int32), "frames": (frames, torch.uint8),
+                                "res": (res, torch.uint8), "out": (out, torch.uint8)})
+    _launch("x3d_jpeg_enc_stuff", lambda: lib().x3d_jpeg_enc_stuff(
+        words.data_ptr(), frames.data_ptr(), nframes, res.data_ptr(), out.data_ptr(), out.numel(), _stream()))
+
+
 def stem_tc_u8_fwd(x: torch.Tensor, mean, std, wc: torch.Tensor, bias: torch.Tensor,
                    norm_value: float = 255.0) -> torch.Tensor:
     """Tensor-core stem with the uint8 input stage fused into its loader; bf16 activations out."""

@@ -4,6 +4,8 @@ dataloader.py:66-91, 150-174 behind `eval.py --tfrecord` / `train.py --use_tfrec
 
   read_records(path)          the records of one GZIP TFRecord file, both CRCs checked
   parse_sequence_example(buf) one record -> TFRecordVideo (label, shape, JPEG bytes of each frame)
+  serialize_sequence_example  JPEG frames + label -> one record (the reference's keys)
+  write_records(path, recs)   one GZIP TFRecord file, both CRCs written
 
 A TFRecordVideo has what video.eval_plan / train_plan need (`shape`) and what video.pack_jpeg reads
 (`jpeg(f)`); its frames are decoded on the device.
@@ -18,7 +20,7 @@ from typing import Iterator, List
 import numpy as np
 
 from . import jpeg as J
-from .tf_bundle import BundleError, _get_varint, _pb_fields, _signed64, crc32c, unmask_crc
+from .tf_bundle import BundleError, _get_varint, _pb_fields, _signed64, crc32c, mask_crc, unmask_crc
 
 CONTEXT_FRAMES = "video/num_frames"
 CONTEXT_LABEL = "video/class/label"
@@ -178,3 +180,56 @@ def read_videos(path: str) -> Iterator[TFRecordVideo]:
     """The videos of one TFRecord file, in file order."""
     for i, rec in enumerate(read_records(path)):
         yield parse_sequence_example(rec, f"{path}:{i}")
+
+
+# ---- writing (the reference's datasets/create_tfrecords.py:48-83, 100-103)
+
+def _varint(n: int) -> bytes:
+    n &= (1 << 64) - 1
+    out = bytearray()
+    while True:
+        b = n & 0x7F
+        n >>= 7
+        if n:
+            out.append(b | 0x80)
+        else:
+            out.append(b)
+            return bytes(out)
+
+
+def _ld(field: int, payload: bytes) -> bytes:
+    """A length-delimited protobuf field."""
+    return _varint(field << 3 | 2) + _varint(len(payload)) + payload
+
+
+def _entry(key: str, value: bytes) -> bytes:
+    """One map<string, message> entry of Features / FeatureLists (field 1)."""
+    return _ld(1, _ld(1, key.encode("utf-8")) + _ld(2, value))
+
+
+def _int64_feature(v: int) -> bytes:
+    return _ld(3, _ld(1, _varint(int(v))))                   # Feature{int64_list{packed value}}
+
+
+def serialize_sequence_example(frames, label: int) -> bytes:
+    """The reference's record: context `video/num_frames` and `video/class/label` (Int64List), feature
+    list `video` with one BytesList of one JPEG per frame, serialised as protobuf does (map entries in
+    key order, as its deterministic serialisation writes them)."""
+    context = _entry(CONTEXT_LABEL, _int64_feature(label)) + _entry(CONTEXT_FRAMES, _int64_feature(len(frames)))
+    video = b"".join(_ld(1, _ld(1, _ld(1, bytes(f)))) for f in frames)
+    return _ld(1, context) + _ld(2, _entry(FRAMES_KEY, video))
+
+
+def write_records(path: str, records, level: int = 6) -> int:
+    """Writes a GZIP TFRecord file (TFRecordWriter with options "GZIP"): per record the uint64 length,
+    its masked CRC-32C, the data and its masked CRC-32C.  Returns the uncompressed bytes written."""
+    _native_crc()
+    n = 0
+    with gzip.open(path, "wb", compresslevel=level) as f:
+        for r in records:
+            head = struct.pack("<Q", len(r))
+            f.write(head + struct.pack("<I", mask_crc(crc32c(head))))
+            f.write(r)
+            f.write(struct.pack("<I", mask_crc(crc32c(r))))
+            n += len(r) + 16
+    return n
