@@ -278,7 +278,11 @@ int x3d_video_clips_u8(const uint8_t* frames, const int64_t* frame_off, const x3
  * parses the headers and rejects everything else on the host).  Every frame of a ragged batch is
  * decoded by one launch per stage.
  *
- * Per frame (component c = 0 luma, 1 Cb, 2 Cr; hs = vs = luma sampling, 1 for chroma):
+ * Motion-JPEG frames (x3d_tf_b200/avi.py) add luma sampling 2x1 (4:2:2) and restart intervals, whose
+ * intervals x3d_jpeg_entropy_rst decodes in parallel.
+ *
+ * Per frame (component c = 0 luma, 1 Cb, 2 Cr; hs, vs = luma sampling, 1 for chroma; an MCU holds the
+ * hs*vs luma blocks in row-major order, then Cb, then Cr: 2x2 = 4 + 2 blocks, 2x1 = 2 side by side + 2):
  *   mcux = ceil(W / (8*hs)), mcuy = ceil(H / (8*vs));  component c has a block grid of
  *   bw_c x bh_c = (mcux*hs_c) x (mcuy*vs_c) blocks, stored component after component, each row-major:
  *   coefficients  int16 [blocks][64], natural order, quantised;  block b of the frame at
@@ -287,7 +291,7 @@ int x3d_video_clips_u8(const uint8_t* frames, const int64_t* frame_off, const x3
  *   output        packed row-major [H][W][3] RGB at out_off (4-byte aligned): exactly what
  *                 x3d_video_clips_u8 reads through frame_off.
  * The descriptors are device data and are NOT checked by the calls; the caller guarantees per frame:
- * 1 <= H, W <= 65535; (hs, vs) = (1, 1) or (2, 2); 0 <= tables < the number of table sets; the segment
+ * 1 <= H, W <= 65535; (hs, vs) = (1, 1), (2, 2) or (2, 1); 0 <= tables < the number of table sets; the segment
  * seg_off .. + seg_len inside `data`; every buffer range above inside its buffer; status < the length
  * of `status`.  Ranges of different frames may not overlap. */
 typedef struct x3d_jpeg_frame {
@@ -335,6 +339,28 @@ enum x3d_jpeg_dct { X3D_JPEG_ISLOW = 0, X3D_JPEG_IFAST = 1 };
  * segment or writes outside its blocks. */
 int x3d_jpeg_entropy(const uint8_t* data, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,
                      int nframes, int16_t* coef, int32_t* status, void* stream);
+/* Stage 1 for frames with a restart interval (DRI != 0): every interval is an independent bit stream whose
+ * DC predictors start at 0, so one launch decodes all intervals of a ragged batch in parallel (one thread
+ * per interval, each with its own bit reader that drops the stuffed 00 after every FF).  An interval
+ * covers MCUs mcu0 .. mcu0 + nmcu - 1 of its frame in raster order; its bytes are data[off .. off + len)
+ * (byte stuffing included, fill bytes and the RSTn / EOI marker that ends it excluded).  Writes every
+ * block of those MCUs into the layout x3d_jpeg_entropy writes (zeros where no coefficient is coded).
+ * An interval that fails raises its frame's status word to its x3d_jpeg_status with atomicMax (so the
+ * result does not depend on the order of the intervals) and leaves its remaining blocks as they were:
+ * the status words of the frames concerned must be zero before the launch.  Never reads outside an
+ * interval or writes outside that interval's blocks.  The host (x3d_tf_b200/jpeg.py parse(mjpeg=True))
+ * guarantees per interval: frame < the number of frames, mcu0 + nmcu <= the frame's MCU count, the byte
+ * range inside `data`; the intervals of a frame cover each of its MCUs once. */
+typedef struct x3d_jpeg_interval {
+  int64_t off;         /* byte offset in `data` */
+  int32_t len;         /* bytes */
+  int32_t frame;       /* index of its x3d_jpeg_frame */
+  int32_t mcu0;        /* first MCU (raster order) */
+  int32_t nmcu;        /* MCUs */
+} x3d_jpeg_interval;
+int x3d_jpeg_entropy_rst(const uint8_t* data, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,
+                         const x3d_jpeg_interval* intervals, int nintervals, int16_t* coef, int32_t* status,
+                         void* stream);
 /* Stage 2, dequantisation and 8x8 inverse DCT into the planes: method X3D_JPEG_ISLOW = jidctint.c
  * jpeg_idct_islow, X3D_JPEG_IFAST = jidctfst.c jpeg_idct_ifast with jddctmgr.c's multiplier table
  * (q * aanscales, descaled by 12 with rounding); both with IDCT_range_limit (wrap-around at RANGE_MASK).
@@ -343,7 +369,9 @@ int x3d_jpeg_idct(const int16_t* coef, const x3d_jpeg_frame* frames, const x3d_j
                   int nframes, int max_blocks, int method, uint8_t* planes, void* stream);
 /* Stage 3, upsampling and colour conversion into the output: chroma of 2x2 frames by jdsample.c
  * h2v2_fancy_upsample (edges replicated at the downsampled extent ceil(W/2) x ceil(H/2); the box
- * h2v2_upsample when ceil(W/2) <= 2, as libjpeg does), then jdcolor.c ycc_rgb_convert.
+ * h2v2_upsample when ceil(W/2) <= 2, as libjpeg does), chroma of 2x1 frames by h2v1_fancy_upsample
+ * (edges replicated at ceil(W/2); the box h2v1_upsample when ceil(W/2) <= 2), then jdcolor.c
+ * ycc_rgb_convert.
  * max_pixels >= H*W of every frame. */
 int x3d_jpeg_color(const uint8_t* planes, const x3d_jpeg_frame* frames, int nframes, int64_t max_pixels,
                    uint8_t* out, void* stream);

@@ -63,6 +63,11 @@ class JpegTables(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class JpegInterval(C.Structure):
+    _fields_ = [("off", C.c_int64), ("len", C.c_int32), ("frame", C.c_int32), ("mcu0", C.c_int32),
+                ("nmcu", C.c_int32)]
+
+
 class JpegEncFrame(C.Structure):
     _fields_ = [("in_off", C.c_int64), ("coef_off", C.c_int64), ("word_off", C.c_int64), ("word_cap", C.c_int64),
                 ("H", C.c_int32), ("W", C.c_int32), ("hs", C.c_int32), ("vs", C.c_int32), ("tables", C.c_int32),
@@ -147,6 +152,7 @@ SIGNATURES = {
     "x3d_eval_views_u8": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 7 + [C.c_void_p]),
     "x3d_video_clips_u8": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p, C.c_void_p]),
     "x3d_jpeg_entropy": (C.c_int, [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3),
+    "x3d_jpeg_entropy_rst": (C.c_int, [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 3),
     "x3d_jpeg_idct": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p] * 2),
     "x3d_jpeg_color": (C.c_int, [C.c_void_p] * 2 + [C.c_int, C.c_int64] + [C.c_void_p] * 2),
     "x3d_jpeg_fdct": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 2 + [C.c_void_p] * 2),

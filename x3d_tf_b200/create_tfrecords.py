@@ -13,6 +13,11 @@ in list order: DIR/shard-00000-of-0000N.tfrecord.gz, ...  `eval.py --tfrecord` a
 `--max_frames` keeps the first K frames of each video (the reference cuts its videos at 10 seconds;
 decoded `.npy` videos carry no frame rate).
 
+With `--mjpeg_videos` the list names Motion-JPEG `.avi` files instead (avi.py).  The frames of a
+shard are decoded on the device (x3d_jpeg_*, IDCT by `--dct_method`, INTEGER_FAST by default as in
+the other drivers) into the packed RGB buffer the decoder writes, and that buffer goes straight to the
+encoder: a transcode from AVI to TFRecords never leaves the device between the two codecs.
+
 The frames of a shard are encoded on the device in one batch and staged through pinned memory; the
 records are serialised, compressed and written on a thread pool while the next shard is encoded.
 At most 2 x `--threads` encoded shards wait for the pool (the oldest is awaited before the next one is
@@ -45,6 +50,25 @@ def _write(path: str, jpegs: List[List[bytes]], labels: List[int], level: int):
     return t1 - t0, time.perf_counter() - t1, raw
 
 
+def _decode_mjpeg(part, max_frames: int, dct_method: str, scratch: dict):
+    """(frames per video, [H, W, 3] uint8 device views of every frame in order) of the Motion-JPEG
+    videos `part`, decoded on the current device in one batch."""
+    import torch
+    from . import avi, video
+    vids = avi.open_videos(part)
+    counts = [min(len(v), max_frames) if max_frames > 0 else len(v) for v in vids]
+    pairs = [(i, f) for i, n in enumerate(counts) for f in range(n)]
+    enc, out_off = video.encoded_frames(vids, pairs, dct_method=dct_method)
+    dec = scratch.setdefault("decode", {})
+    out, status = enc.decode(torch.device("cuda", torch.cuda.current_device()), dec)
+    enc.check(status.cpu().numpy())
+    frames = []
+    for (i, _), o in zip(pairs, out_off):
+        _, H, W, _ = vids[i].shape
+        frames.append(out[int(o):int(o) + H * W * 3].view(H, W, 3))
+    return counts, frames
+
+
 def run(argv: Optional[List[str]] = None) -> dict:
     ap = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     ap.add_argument("--file_list", required=True, help="text file: '<video.npy> <label>' per video")
@@ -55,6 +79,9 @@ def run(argv: Optional[List[str]] = None) -> dict:
     ap.add_argument("--max_frames", type=int, default=0, help="keep the first K frames of each video (0: all)")
     ap.add_argument("--gzip_level", type=int, default=6)
     ap.add_argument("--threads", type=int, default=min(16, os.cpu_count() or 1))
+    ap.add_argument("--mjpeg_videos", action="store_true", help="list lines name Motion-JPEG .avi videos")
+    ap.add_argument("--dct_method", default="INTEGER_FAST", choices=["INTEGER_FAST", "INTEGER_ACCURATE"],
+                    help="IDCT of the JPEG decoder for --mjpeg_videos (tf.io.decode_jpeg's names)")
     a = ap.parse_args(argv)
     import torch
     if not torch.cuda.is_available():
@@ -78,16 +105,20 @@ def run(argv: Optional[List[str]] = None) -> dict:
             while len(pending) >= max_pending:
                 done.append(pending.popleft().result())
             part = items[s * a.videos_per_file:(s + 1) * a.videos_per_file]
-            videos = [load_video(p) for p, _ in part]
-            if a.max_frames > 0:
-                videos = [v[:a.max_frames] for v in videos]
             t1 = time.perf_counter()
-            flat = J.encode_frames([f for v in videos for f in v], a.quality, a.chroma, scratch)
+            if a.mjpeg_videos:
+                counts, frame_list = _decode_mjpeg(part, a.max_frames, a.dct_method, scratch)
+            else:
+                videos = [load_video(p) for p, _ in part]
+                if a.max_frames > 0:
+                    videos = [v[:a.max_frames] for v in videos]
+                counts, frame_list = [len(v) for v in videos], [f for v in videos for f in v]
+            flat = J.encode_frames(frame_list, a.quality, a.chroma, scratch)
             encode_s += time.perf_counter() - t1
             jpegs, k = [], 0
-            for v in videos:
-                jpegs.append(flat[k:k + len(v)])
-                k += len(v)
+            for n in counts:
+                jpegs.append(flat[k:k + n])
+                k += n
             frames += len(flat)
             jpeg_bytes += sum(len(b) for b in flat)
             pending.append(pool.submit(_write, shard_name(a.out_dir, s, nshards), jpegs, [lab for _, lab in part],

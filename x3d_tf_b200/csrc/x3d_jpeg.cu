@@ -2,8 +2,9 @@
 // dataloader.py:66-91, 150-174), in three stages that reproduce libjpeg-turbo's decompressor in its
 // default libjpeg-6b mode bit for bit (pure integer arithmetic):
 //   x3d_jpeg_entropy  Huffman decoding (jdhuff.c)                  -> int16 coefficient blocks
+//   x3d_jpeg_entropy_rst  the same for frames with restart intervals, one thread per interval
 //   x3d_jpeg_idct     dequantisation + jidctint.c / jidctfst.c     -> per-component sample planes
-//   x3d_jpeg_color    jdsample.c h2v2_fancy_upsample + jdcolor.c   -> packed [H][W][3] RGB frames
+//   x3d_jpeg_color    jdsample.c h2v2 / h2v1_fancy_upsample + jdcolor.c -> packed [H][W][3] RGB frames
 // Layouts and preconditions: include/x3d_b200.h.
 #include "common.cuh"
 
@@ -220,6 +221,136 @@ entropy_kernel(const uint8_t* __restrict__ data, const x3d_jpeg_frame* __restric
 }
 
 // ---------------------------------------------------------------------------------------------
+// Stage 1 for restart intervals: one thread per interval, reading its bytes straight from global
+// memory (each thread walks its own range sequentially, so the lines it touches stay in L1) and
+// dropping the 00 stuffed after every FF.  A block is decoded into the thread's zeroed slot in shared
+// memory and stored as eight 16-byte words.  The Huffman tables are read through the read-only cache:
+// the intervals of one CTA may belong to frames with different tables.
+constexpr int kRstThreads = 64;
+
+struct RstReader {
+  uint64_t acc;        // MSB-aligned
+  int nbits;
+  int32_t pos;         // next byte of the interval
+  int32_t zeros;       // zero bytes appended past the interval's end
+  const uint8_t* p;
+  int32_t len;
+
+  __device__ __forceinline__ void fill() {
+    while (nbits <= 56) {
+      uint32_t b = 0;
+      if (pos < len) {
+        b = __ldg(p + pos);
+        pos += (b == 0xFF) ? 2 : 1;                 // FF 00 -> FF (a range never ends inside FF 00)
+      } else {
+        ++zeros;
+      }
+      acc |= static_cast<uint64_t>(b) << (56 - nbits);
+      nbits += 8;
+    }
+  }
+  __device__ __forceinline__ uint32_t peek(int n) const { return static_cast<uint32_t>(acc >> (64 - n)); }
+  __device__ __forceinline__ void skip(int n) { acc <<= n; nbits -= n; }
+  // bits were taken from the zeros past the end
+  __device__ __forceinline__ bool overran() const { return zeros * 8 > nbits; }
+};
+
+__device__ __forceinline__ int rst_huff_decode(RstReader& br, const x3d_jpeg_huff* __restrict__ h) {
+  br.fill();
+  const uint32_t look = __ldg(&h->lookup[br.peek(8)]);
+  int l = look >> 8;
+  if (l <= 8) {
+    br.skip(l);
+    return look & 0xff;
+  }
+  int32_t code = static_cast<int32_t>(br.peek(9));
+  l = 9;
+  while (l <= 16 && code > __ldg(&h->maxcode[l])) {
+    ++l;
+    code = static_cast<int32_t>(br.peek(l));
+  }
+  if (l > 16) return -1;
+  br.skip(l);
+  return __ldg(&h->huffval[(code + __ldg(&h->valoffset[l])) & 0xff]);
+}
+
+__device__ __forceinline__ int rst_get_bits(RstReader& br, int s) {
+  br.fill();
+  const int r = static_cast<int>(br.peek(s));
+  br.skip(s);
+  return r;
+}
+
+__global__ void __launch_bounds__(kRstThreads)
+entropy_rst_kernel(const uint8_t* __restrict__ data, const x3d_jpeg_frame* __restrict__ frames,
+                   const x3d_jpeg_tables* __restrict__ tables, const x3d_jpeg_interval* __restrict__ intervals,
+                   int nintervals, int16_t* __restrict__ coef, int32_t* __restrict__ status) {
+  __shared__ __align__(16) int16_t blk_s[kRstThreads][64];
+  const int i = blockIdx.x * kRstThreads + threadIdx.x;
+  int4* slot = reinterpret_cast<int4*>(blk_s[threadIdx.x]);
+#pragma unroll
+  for (int q = 0; q < 8; ++q) slot[q] = make_int4(0, 0, 0, 0);
+  if (i >= nintervals) return;
+  const x3d_jpeg_interval iv = intervals[i];
+  const x3d_jpeg_frame fr = frames[iv.frame];
+  const x3d_jpeg_tables* tb = tables + fr.tables;
+  const int hs = fr.hs, vs = fr.vs;
+  const int mcux = (fr.W + 8 * hs - 1) / (8 * hs), mcuy = (fr.H + 8 * vs - 1) / (8 * vs);
+  const int nluma = hs * vs, nb = nluma + 2;
+  const int bw0 = mcux * hs;
+  const int64_t base0 = fr.coef_off, base1 = base0 + static_cast<int64_t>(mcux) * hs * mcuy * vs;
+  const int64_t base2 = base1 + static_cast<int64_t>(mcux) * mcuy;
+  // table ids of the three components, one bit each (no per-thread arrays: they would live in local memory)
+  const int dct = (tb->comp_dc[0] & 1) | (tb->comp_dc[1] & 1) << 1 | (tb->comp_dc[2] & 1) << 2;
+  const int act = (tb->comp_ac[0] & 1) | (tb->comp_ac[1] & 1) << 1 | (tb->comp_ac[2] & 1) << 2;
+  int16_t* blk = blk_s[threadIdx.x];
+  RstReader br{0ull, 0, 0, 0, data + iv.off, iv.len};
+  int pred0 = 0, pred1 = 0, pred2 = 0;       // DC predictors restart at 0 in every interval
+  int err = X3D_JPEG_OK;
+  for (int m = iv.mcu0; m < iv.mcu0 + iv.nmcu && err == X3D_JPEG_OK; ++m) {
+    const int my = m / mcux, mx = m - my * mcux;
+    for (int b = 0; b < nb; ++b) {
+      const int c = b < nluma ? 0 : b - nluma + 1;
+      int s = rst_huff_decode(br, &tb->dc[(dct >> c) & 1]);
+      if (s < 0) { err = X3D_JPEG_BAD_CODE; break; }
+      if (s) s = huff_extend(rst_get_bits(br, s), s);
+      const int pred = static_cast<int>(static_cast<uint32_t>(c == 0 ? pred0 : (c == 1 ? pred1 : pred2)) +
+                                        static_cast<uint32_t>(s));
+      if (c == 0) pred0 = pred; else if (c == 1) pred1 = pred; else pred2 = pred;
+      blk[0] = static_cast<int16_t>(pred);
+      const x3d_jpeg_huff* at = &tb->ac[(act >> c) & 1];
+      for (int k = 1; k < 64; ++k) {
+        s = rst_huff_decode(br, at);
+        if (s < 0) { err = X3D_JPEG_BAD_CODE; break; }
+        const int r = s >> 4;
+        s &= 15;
+        if (s) {
+          k += r;
+          if (k > 63) { err = X3D_JPEG_BAD_RUN; break; }
+          blk[kNatural[k]] = static_cast<int16_t>(huff_extend(rst_get_bits(br, s), s));
+        } else {
+          if (r != 15) break;                                       // EOB
+          k += 15;
+          if (k > 63) { err = X3D_JPEG_BAD_RUN; break; }
+        }
+      }
+      if (err == X3D_JPEG_OK && br.overran()) err = X3D_JPEG_SHORT_DATA;
+      if (err != X3D_JPEG_OK) break;
+      int64_t blkno;
+      if (b < nluma) blkno = base0 + static_cast<int64_t>(my * vs + b / hs) * bw0 + mx * hs + b % hs;
+      else blkno = (b == nluma ? base1 : base2) + static_cast<int64_t>(my) * mcux + mx;
+      int4* dst = reinterpret_cast<int4*>(coef + blkno * 64);
+#pragma unroll
+      for (int q = 0; q < 8; ++q) {
+        dst[q] = slot[q];
+        slot[q] = make_int4(0, 0, 0, 0);
+      }
+    }
+  }
+  if (err != X3D_JPEG_OK) atomicMax(status + fr.status, err);
+}
+
+// ---------------------------------------------------------------------------------------------
 // Stage 2: IDCT.  A CTA takes 32 consecutive blocks of one frame; thread (block, r) runs column r of
 // pass 1 and row r of pass 2 and stores the row's 8 samples with one 8-byte store.  The arithmetic
 // is libjpeg's with JLONG = 64-bit, so even pathological coefficients give libjpeg's result.
@@ -365,6 +496,16 @@ struct Planes {
   int w, dw, dh;        // plane row pitch, downsampled extent
 };
 
+// chroma sample at output pixel (y, x) of a 2x1 frame: jdsample.c h2v1_fancy_upsample (fancy = 1) or
+// h2v1_upsample (fancy = 0, two columns or fewer)
+__device__ __forceinline__ int chroma_h2v1(const Planes& pl, int y, int x, bool fancy) {
+  const uint8_t* r = pl.p + static_cast<int64_t>(y) * pl.w;
+  const int j = x >> 1;
+  if (!fancy) return r[j];
+  if (x & 1) return j == pl.dw - 1 ? r[j] : (r[j] * 3 + r[j + 1] + 2) >> 2;
+  return j == 0 ? r[0] : (r[j] * 3 + r[j - 1] + 1) >> 2;
+}
+
 // chroma sample at output pixel (y, x): jdsample.c h2v2_fancy_upsample (fancy = 1), h2v2_upsample
 // (fancy = 0, two columns or fewer), or the sample itself (1x1 luma)
 __device__ __forceinline__ int chroma(const Planes& pl, int y, int x, int up, bool fancy) {
@@ -392,12 +533,13 @@ color_kernel(const uint8_t* __restrict__ planes, const x3d_jpeg_frame* __restric
   const int mcux = (fr.W + 8 * hs - 1) / (8 * hs), mcuy = (fr.H + 8 * vs - 1) / (8 * vs);
   const int w0 = mcux * hs * 8, w1 = mcux * 8;
   const int up = hs == 2;
+  const bool h2v1 = up && vs == 1;                 // 4:2:2 (Motion-JPEG frames)
   Planes cb, cr;
   cb.p = planes + fr.plane_off + static_cast<int64_t>(w0) * mcuy * vs * 8;
   cr.p = cb.p + static_cast<int64_t>(w1) * mcuy * 8;
   cb.w = cr.w = w1;
   cb.dw = cr.dw = up ? (fr.W + 1) >> 1 : fr.W;
-  cb.dh = cr.dh = up ? (fr.H + 1) >> 1 : fr.H;
+  cb.dh = cr.dh = up && !h2v1 ? (fr.H + 1) >> 1 : fr.H;
   const bool fancy = cb.dw > 2;
   const uint8_t* yp = planes + fr.plane_off;
   uint32_t v[12];
@@ -406,7 +548,8 @@ color_kernel(const uint8_t* __restrict__ planes, const x3d_jpeg_frame* __restric
     const int64_t p = min(p0 + k, npix - 1);
     const int y = static_cast<int>(p / fr.W), x = static_cast<int>(p - static_cast<int64_t>(y) * fr.W);
     const int Y = yp[static_cast<int64_t>(y) * w0 + x];
-    const int Cb = chroma(cb, y, x, up, fancy) - 128, Cr = chroma(cr, y, x, up, fancy) - 128;
+    const int Cb = (h2v1 ? chroma_h2v1(cb, y, x, fancy) : chroma(cb, y, x, up, fancy)) - 128;
+    const int Cr = (h2v1 ? chroma_h2v1(cr, y, x, fancy) : chroma(cr, y, x, up, fancy)) - 128;
     v[3 * k + 0] = clamp255(Y + ((91881 * Cr + 32768) >> 16));
     v[3 * k + 1] = clamp255(Y + ((-22554 * Cb + 32768 - 46802 * Cr) >> 16));
     v[3 * k + 2] = clamp255(Y + ((116130 * Cb + 32768) >> 16));
@@ -438,6 +581,23 @@ extern "C" int x3d_jpeg_entropy(const uint8_t* data, const x3d_jpeg_frame* frame
               X3D_ERR_INVALID_ARG, "x3d_jpeg_entropy: coef must be 16-byte, frames 8-byte, tables/status 4-byte aligned");
   jpeg::entropy_kernel<<<nframes, 32, 0, static_cast<cudaStream_t>(stream)>>>(data, frames, tables, coef, status);
   return check_launch("x3d_jpeg_entropy");
+}
+
+extern "C" int x3d_jpeg_entropy_rst(const uint8_t* data, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,
+                                    const x3d_jpeg_interval* intervals, int nintervals, int16_t* coef, int32_t* status,
+                                    void* stream) {
+  X3D_REQUIRE(data && frames && tables && intervals && coef && status, X3D_ERR_INVALID_ARG,
+              "x3d_jpeg_entropy_rst: null pointer");
+  X3D_REQUIRE(nintervals > 0, X3D_ERR_INVALID_ARG, "x3d_jpeg_entropy_rst: nintervals=%d", nintervals);
+  X3D_REQUIRE((reinterpret_cast<uintptr_t>(coef) & 15) == 0 && (reinterpret_cast<uintptr_t>(frames) & 7) == 0 &&
+              (reinterpret_cast<uintptr_t>(intervals) & 7) == 0 && (reinterpret_cast<uintptr_t>(tables) & 3) == 0 &&
+              (reinterpret_cast<uintptr_t>(status) & 3) == 0,
+              X3D_ERR_INVALID_ARG,
+              "x3d_jpeg_entropy_rst: coef must be 16-byte, frames/intervals 8-byte, tables/status 4-byte aligned");
+  const int grid = (nintervals + jpeg::kRstThreads - 1) / jpeg::kRstThreads;
+  jpeg::entropy_rst_kernel<<<grid, jpeg::kRstThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      data, frames, tables, intervals, nintervals, coef, status);
+  return check_launch("x3d_jpeg_entropy_rst");
 }
 
 extern "C" int x3d_jpeg_idct(const int16_t* coef, const x3d_jpeg_frame* frames, const x3d_jpeg_tables* tables,

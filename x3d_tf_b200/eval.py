@@ -21,7 +21,10 @@ x3d_video_clips_u8), and only the frames the views sample are read and copied.  
 (`tfrecord.py`; taken in sorted order, ranks get contiguous blocks of files, records are read in
 file order): the JPEG frames the views sample are decoded on the device (x3d_jpeg_*) and then go
 through the same clip kernel.  `--dct_method` picks the IDCT as TF's decode_jpeg names it:
-INTEGER_FAST (TF 2.4's default for dct_method='') or INTEGER_ACCURATE.  `--synthetic V` evaluates V
+INTEGER_FAST (TF 2.4's default for dct_method='') or INTEGER_ACCURATE.  With `--mjpeg_videos` the
+list lines name Motion-JPEG `.avi` files, the reference's default `<video> <label>` lists (`avi.py`):
+the same plans and sharding as `--decoded_videos`, and only the JPEG frames the views sample are read
+from the files and decoded on the device.  `--synthetic V` evaluates V
 seeded random videos instead (no files needed).
 """
 from __future__ import annotations
@@ -81,6 +84,15 @@ def video_batches(items: List[Tuple[str, int]], videos_per_batch: int, cfg):
                np.asarray([lab for _, lab in chunk], np.int32))
 
 
+def mjpeg_batches(items: List[Tuple[str, int]], videos_per_batch: int, cfg, dct_method: str = "INTEGER_FAST"):
+    """Batches of Motion-JPEG AVI videos as video.VideoBatch of JPEG frames."""
+    from . import avi, video
+    for i in range(0, len(items), videos_per_batch):
+        chunk = items[i:i + videos_per_batch]
+        yield (video.eval_batch(avi.open_videos(chunk), cfg, dct_method),
+               np.asarray([lab for _, lab in chunk], np.int32))
+
+
 def tfrecord_files(pattern: str) -> List[str]:
     """The GZIP TFRecord files a glob names, sorted."""
     files = sorted(glob.glob(pattern))
@@ -132,6 +144,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
                     help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
     ap.add_argument("--tfrecord", action="store_true",
                     help="--test_file_pattern is a glob of GZIP TFRecord files (JPEG frames, decoded on the device)")
+    ap.add_argument("--mjpeg_videos", action="store_true",
+                    help="list lines name Motion-JPEG .avi videos (JPEG frames decoded on the device)")
     ap.add_argument("--dct_method", default="INTEGER_FAST", choices=["INTEGER_FAST", "INTEGER_ACCURATE"],
                     help="IDCT of the JPEG decoder (tf.io.decode_jpeg's names; INTEGER_FAST is its default)")
     ap.add_argument("--gpus", type=int, default=1)
@@ -146,8 +160,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     a = ap.parse_args(argv)
     if not a.test_file_pattern and not a.synthetic:
         ap.error("one of --test_file_pattern / --synthetic is required")
-    if a.tfrecord and a.decoded_videos:
-        ap.error("--tfrecord and --decoded_videos are mutually exclusive")
+    if a.tfrecord + a.decoded_videos + a.mjpeg_videos > 1:
+        ap.error("--tfrecord, --decoded_videos and --mjpeg_videos are mutually exclusive")
     cfg = load_cfg(a.cfg)
     if not os.path.isdir(a.model_folder):
         raise NotADirectoryError(a.model_folder)          # eval.py:36-37
@@ -192,8 +206,12 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     else:
         items = read_file_list(a.test_file_pattern)
         lo, hi = shard.shard_range(len(items), world, rank)
-        data = (video_batches(items[lo:hi], vpb, cfg) if a.decoded_videos
-                else file_batches(items[lo:hi], vpb, num_preds))
+        if a.mjpeg_videos:
+            data = mjpeg_batches(items[lo:hi], vpb, cfg, a.dct_method)
+        elif a.decoded_videos:
+            data = video_batches(items[lo:hi], vpb, cfg)
+        else:
+            data = file_batches(items[lo:hi], vpb, num_preds)
     res = model.evaluate(data, verbose=1 if rank == 0 else 0)
     if rank == 0:
         print(f"\nloss: {res['loss']:.4f} - acc: {res['acc']:.4f} - top_5_acc: {res['top_5_acc']:.4f} "

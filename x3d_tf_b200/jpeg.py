@@ -11,11 +11,21 @@ device.
 The frames of one encoder run share their header, so `parse` caches the parsed tables by the header
 bytes (everything before the entropy-coded segment); a batch then carries one table set per distinct
 header.
+
+`parse(buf, mjpeg=True)` is the opt-in for the frames of Motion-JPEG videos (avi.py; TFRecord reading
+never uses it).  It accepts, on top of the above:
+  - a restart interval (DRI != 0): the RSTn markers must cycle RST0..RST7 and there must be exactly
+    ceil(MCUs / Ri) - 1 of them before EOI; JpegFrame.intervals gives each interval's byte range
+    (byte stuffing included, fill bytes and the marker excluded), which the device decodes in parallel
+    (x3d_jpeg_entropy_rst);
+  - luma sampling 2x1 (4:2:2), chroma 1x1;
+  - no DHT segment: the missing Huffman tables of ids 0 and 1 are the standard (Annex K) ones, as
+    libjpeg-turbo's decompressor sets them for Motion-JPEG (jstdhuff.c std_huff_tables).
 """
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 
@@ -30,6 +40,7 @@ ZIGZAG = np.array([
 LOOKAHEAD = 8
 TABLES_DTYPE = np.dtype(_lib.JpegTables)
 FRAME_DTYPE = np.dtype(_lib.JpegFrame)
+INTERVAL_DTYPE = np.dtype(_lib.JpegInterval)
 
 _SOF_REASON = {0xC1: "extended sequential (SOF1)", 0xC2: "progressive (SOF2)", 0xC3: "lossless (SOF3)",
                0xC5: "hierarchical (SOF5)", 0xC6: "hierarchical progressive (SOF6)",
@@ -64,6 +75,11 @@ class JpegHeader:
     ac: Tuple[DerivedTable, ...]
     scan_off: int                          # offset of the entropy-coded segment = header length
     tables: np.ndarray                     # the x3d_jpeg_tables record the device reads
+    ri: int = 0                            # restart interval in MCUs (0: none; mjpeg parsing only)
+
+    @property
+    def mcus(self) -> int:
+        return -(-self.W // (8 * self.hs)) * -(-self.H // (8 * self.vs))
 
 
 @dataclass(frozen=True)
@@ -71,6 +87,8 @@ class JpegFrame:
     header: JpegHeader
     seg_off: int                           # the entropy-coded segment (byte stuffing included)
     seg_len: int
+    intervals: Optional[np.ndarray] = None   # [n, 2] int64 (offset in buf, length) of each restart
+                                             # interval when header.ri != 0, else None
 
 
 def derive_table(bits, huffval, is_dc: bool) -> DerivedTable:
@@ -141,8 +159,9 @@ def _header_end(buf) -> int:
             return pos
 
 
-def _parse_header(hdr) -> JpegHeader:
+def _parse_header(hdr, mjpeg: bool = False) -> JpegHeader:
     q: Dict[int, np.ndarray] = {}
+    ri = 0
     huff: Dict[Tuple[int, int], DerivedTable] = {}
     sof = scan = None
     adobe = jfif = False
@@ -205,8 +224,11 @@ def _parse_header(hdr) -> JpegHeader:
         elif m == 0xCC:
             raise ValueError("arithmetic coding conditioning (DAC): only Huffman coding is supported")
         elif m == 0xDD:
-            if len(seg) < 2 or _u16(seg, 0) != 0:
+            if len(seg) < 2:
+                raise ValueError("malformed DRI segment")
+            if _u16(seg, 0) != 0 and not mjpeg:
                 raise ValueError("restart interval (DRI != 0) is not supported")
+            ri = _u16(seg, 0)
         elif m == 0xDA:
             ns = seg[0] if seg else 0
             if ns != 3:
@@ -229,15 +251,22 @@ def _parse_header(hdr) -> JpegHeader:
     (hs, vs), chroma = comps[0][1:3], [c[1:3] for c in comps[1:]]
     if any(c != (1, 1) for c in chroma):
         raise ValueError(f"chroma sampling {chroma}: only 1x1 chroma is supported")
-    if (hs, vs) == (2, 1) or (hs, vs) == (1, 2):
+    if mjpeg and (hs, vs) == (2, 1):
+        pass                                                  # 4:2:2, Motion-JPEG frames only
+    elif (hs, vs) == (2, 1) or (hs, vs) == (1, 2):
         raise ValueError(f"4:2:2 / 4:4:0 JPEG (luma sampling {hs}x{vs}): only 4:2:0 and 4:4:4 are supported")
-    if (hs, vs) not in ((1, 1), (2, 2)):
+    elif (hs, vs) not in ((1, 1), (2, 2)):
         raise ValueError(f"luma sampling {hs}x{vs}: only 2x2 (4:2:0) and 1x1 (4:4:4) are supported")
     if [s[0] for s in scan] != ids:
         raise ValueError("the scan's components are not the frame's in frame order")
     comp_q = tuple(int(c[3]) for c in comps)
     comp_dc = tuple(int(s[1]) for s in scan)
     comp_ac = tuple(int(s[2]) for s in scan)
+    if mjpeg:
+        for k, (bits, vals) in enumerate(STD_HUFF):       # DC0, AC0, DC1, AC1 where the frame has none
+            key = (k & 1, k >> 1)
+            if key not in huff:
+                huff[key] = _std_table(k)
     for k in range(3):
         if comp_q[k] not in q:
             raise ValueError(f"component {k}: quantisation table {comp_q[k]} is not defined")
@@ -256,31 +285,76 @@ def _parse_header(hdr) -> JpegHeader:
                     rec[name][f][i] = getattr(t, f)
     rec["q"] = qt
     rec["comp_q"], rec["comp_dc"], rec["comp_ac"] = comp_q, comp_dc, comp_ac
-    return JpegHeader(H, W, hs, vs, qt, comp_q, comp_dc, comp_ac, dc, ac, len(hdr), rec)
+    return JpegHeader(H, W, hs, vs, qt, comp_q, comp_dc, comp_ac, dc, ac, len(hdr), rec, ri)
 
 
 _cache: Dict[bytes, JpegHeader] = {}
+_mjpeg_cache: Dict[bytes, JpegHeader] = {}
+_std_tables: Dict[int, DerivedTable] = {}
 
 
-def parse_header(buf) -> JpegHeader:
-    """The header of one JPEG frame (cached by its bytes)."""
+def _std_table(k: int) -> DerivedTable:
+    """STD_HUFF[k] derived (k: 0 DC0, 1 AC0, 2 DC1, 3 AC1)."""
+    t = _std_tables.get(k)
+    if t is None:
+        bits, vals = STD_HUFF[k]
+        t = _std_tables[k] = derive_table([0] + bits, bytes(vals), k % 2 == 0)
+    return t
+
+
+def parse_header(buf, mjpeg: bool = False) -> JpegHeader:
+    """The header of one JPEG frame (cached by its bytes; `mjpeg`: module docstring)."""
     end = _header_end(buf)
     key = bytes(buf[:end])
-    h = _cache.get(key)
+    cache = _mjpeg_cache if mjpeg else _cache
+    h = cache.get(key)
     if h is None:
-        h = _parse_header(key)
-        if len(_cache) > 4096:
-            _cache.clear()
-        _cache[key] = h
+        h = _parse_header(key, mjpeg)
+        if len(cache) > 4096:
+            cache.clear()
+        cache[key] = h
     return h
 
 
-def parse(buf) -> JpegFrame:
+def _intervals(a: np.ndarray, h: JpegHeader, base: int) -> Tuple[int, np.ndarray]:
+    """(segment length up to EOI's fill bytes, [n, 2] (offset, length) of each restart interval) of
+    the entropy-coded bytes `a` (starting at offset `base` of the frame)."""
+    n = -(-h.mcus // h.ri)
+    pos = np.flatnonzero((a[:-1] == 0xFF) & (a[1:] != 0x00) & (a[1:] != 0xFF))     # a marker at each
+    codes = a[pos[:n] + 1]
+    if pos.size < n or codes[-1] != 0xD9:
+        found = int(np.count_nonzero((codes >= 0xD0) & (codes <= 0xD7)))
+        raise ValueError(f"{found} restart markers before the end of the scan: "
+                         f"{n - 1} expected ({h.mcus} MCUs, restart interval {h.ri})")
+    want = 0xD0 + np.arange(n - 1) % 8
+    bad = np.flatnonzero(codes[:-1] != want)
+    if bad.size:
+        i = int(bad[0])
+        raise ValueError(f"marker 0x{int(codes[i]):02X} where RST{i % 8} (restart interval {i + 1} of {n}) "
+                         "was expected")
+    ends = pos[:n].copy()
+    for i in np.flatnonzero(a[np.maximum(ends - 1, 0)] == 0xFF):           # fill bytes before a marker
+        while ends[i] > 0 and a[ends[i] - 1] == 0xFF:
+            ends[i] -= 1
+    starts = np.concatenate([[0], pos[:n - 1] + 2])
+    if (ends < starts).any():
+        raise ValueError("malformed restart interval")
+    iv = np.stack([starts + base, ends - starts], 1).astype(np.int64)
+    return int(ends[-1]), iv
+
+
+def parse(buf, mjpeg: bool = False) -> JpegFrame:
     """Header and entropy-coded segment of one frame.  The segment runs up to the first marker
     (0xFF followed by a byte other than 0x00), which must be EOI: restart markers, a second scan or
-    a DNL are rejected."""
-    h = parse_header(buf)
+    a DNL are rejected.  With `mjpeg` (module docstring), a frame with a restart interval has its
+    segment up to EOI and the byte range of every interval."""
+    h = parse_header(buf, mjpeg)
     a = np.frombuffer(buf, np.uint8)[h.scan_off:]
+    if h.ri:
+        if a.size < 2:
+            raise ValueError("JPEG entropy-coded segment without an end marker")
+        seg_len, iv = _intervals(a, h, h.scan_off)
+        return JpegFrame(h, h.scan_off, seg_len, iv)
     ff = np.flatnonzero(a[:-1] == 0xFF)
     ff = ff[a[ff + 1] != 0]
     if ff.size == 0:

@@ -172,6 +172,25 @@ def jpeg_entropy(data: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor,
         data.data_ptr(), frames.data_ptr(), tables.data_ptr(), nframes, coef.data_ptr(), status.data_ptr(), _stream()))
 
 
+def jpeg_entropy_rst(data: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, intervals: torch.Tensor,
+                     nintervals: int, coef: torch.Tensor, status: torch.Tensor, status_lo: int, status_hi: int) -> None:
+    """x3d_jpeg_entropy_rst: Huffman-decode `nintervals` restart intervals (`intervals`: the
+    x3d_jpeg_interval records as a raw uint8 device buffer, validated on the host by video.pack_jpeg)
+    into `coef`.  The kernel only raises status words (atomicMax), so the words status[status_lo:
+    status_hi] of the frames the intervals belong to are cleared on the stream first."""
+    for t, name in ((data, "data"), (frames, "frames"), (tables, "tables"), (intervals, "intervals"),
+                    (coef, "coef"), (status, "status")):
+        _req(t, name)
+    if coef.dtype != torch.int16 or status.dtype != torch.int32:
+        raise TypeError("jpeg_entropy_rst: coef int16, status int32")
+    if not 0 <= status_lo <= status_hi <= status.numel():
+        raise ValueError(f"jpeg_entropy_rst: status words {status_lo}..{status_hi} of {status.numel()}")
+    status[status_lo:status_hi].zero_()
+    _launch("x3d_jpeg_entropy_rst", lambda: lib().x3d_jpeg_entropy_rst(
+        data.data_ptr(), frames.data_ptr(), tables.data_ptr(), intervals.data_ptr(), nintervals, coef.data_ptr(),
+        status.data_ptr(), _stream()))
+
+
 def jpeg_idct(coef: torch.Tensor, frames: torch.Tensor, tables: torch.Tensor, nframes: int, max_blocks: int,
               method: int, planes: torch.Tensor) -> None:
     """x3d_jpeg_idct: dequantise + 8x8 IDCT (method _lib.X3D_JPEG_ISLOW / X3D_JPEG_IFAST) into `planes`."""

@@ -22,7 +22,10 @@ slot draws one random clip of its video (temporal start, short-side scale jitter
 `--use_tfrecord` (the reference's flag), globs of the reference's GZIP TFRecord files: the file list
 is shuffled per epoch with the epoch seed (the same on every rank), rank r reads files r::world,
 records stream through a shuffle buffer of 16 x the per-rank batch (dataloader.py:158-159) and
-repeat as needed, and the sampled JPEG frames are decoded on the device (x3d_jpeg_*);
+repeat as needed, and the sampled JPEG frames are decoded on the device (x3d_jpeg_*); or, with
+`--mjpeg_videos`, lists of Motion-JPEG `.avi` files (the reference's default `<video> <label>` lists,
+`avi.py`), drawn as with `--decoded_videos`, whose sampled JPEG frames are read and decoded on the
+device;
 `--synthetic N` trains on N seeded random clips per epoch instead.  W&B / TensorBoard callbacks are
 not reproduced; the per-epoch log line carries the same quantities Keras prints.
 """
@@ -87,15 +90,18 @@ def file_clip_batches(items: List[Tuple[str, int]], gbatch: int, steps: int, see
 
 
 def video_clip_batches(items: List[Tuple[str, int]], gbatch: int, steps: int, seed: int, cfg, rank: int = 0,
-                       world: int = 1, crop_size: int = 0):
+                       world: int = 1, crop_size: int = 0, mjpeg: bool = False, dct_method: str = "INTEGER_FAST"):
     """This rank's slice of every global batch as a video.VideoBatch: one random clip per listed
-    decoded video, the random numbers from video.train_rng(seed, rank) (per epoch and rank)."""
-    from . import video
+    decoded video (`mjpeg`: Motion-JPEG AVI video), the random numbers from video.train_rng(seed,
+    rank) (per epoch and rank)."""
+    from . import avi, video
     batch = gbatch // world
     rng = video.train_rng(seed, rank)
     for idx in global_batch_indices(len(items), gbatch, steps, seed):
         mine = idx[rank * batch:(rank + 1) * batch]
-        vb = video.train_batch([video.load_video(items[j][0]) for j in mine], cfg, rng, crop_size)
+        vids = (avi.open_videos([items[j] for j in mine]) if mjpeg
+                else [video.load_video(items[j][0]) for j in mine])
+        vb = video.train_batch(vids, cfg, rng, crop_size, dct_method)
         yield vb, np.asarray([items[j][1] for j in mine], np.int32)
 
 
@@ -163,6 +169,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
                     help="list lines name decoded videos [F,H,W,3] uint8 (.npy, any size): clips are built on the device")
     ap.add_argument("--use_tfrecord", action="store_true",
                     help="the file patterns are globs of GZIP TFRecord files (JPEG frames, decoded on the device)")
+    ap.add_argument("--mjpeg_videos", action="store_true",
+                    help="list lines name Motion-JPEG .avi videos (JPEG frames decoded on the device)")
     ap.add_argument("--dct_method", default="INTEGER_FAST", choices=["INTEGER_FAST", "INTEGER_ACCURATE"],
                     help="IDCT of the JPEG decoder (tf.io.decode_jpeg's names; INTEGER_FAST is its default)")
     ap.add_argument("--model_dir", required=True)
@@ -179,8 +187,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     a = ap.parse_args(argv)
     if not a.train_file_pattern and not a.synthetic:
         ap.error("one of --train_file_pattern / --synthetic is required")
-    if a.use_tfrecord and a.decoded_videos:
-        ap.error("--use_tfrecord and --decoded_videos are mutually exclusive")
+    if a.use_tfrecord + a.decoded_videos + a.mjpeg_videos > 1:
+        ap.error("--use_tfrecord, --decoded_videos and --mjpeg_videos are mutually exclusive")
     if a.config.endswith(".yaml"):
         cfg = get_default_config(); cfg.merge_from_file(a.config); cfg.freeze()
     else:
@@ -208,7 +216,7 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     from .arch import build_arch
     from .model import X3D, keras_default_weights, reset_block_counters
     from .training import X3DTrainer
-    from .eval import file_batches, tfrecord_batches, tfrecord_files, video_batches
+    from .eval import file_batches, mjpeg_batches, tfrecord_batches, tfrecord_files, video_batches
     from .video import VideoBatch
 
     tr = X3DTrainer(cfg, device=dev, world=world, rank=rank)
@@ -249,8 +257,9 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
         if items is not None and a.use_tfrecord:
             data = tfrecord_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size,
                                          a.dct_method)
-        elif items is not None and a.decoded_videos:
-            data = video_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size)
+        elif items is not None and (a.decoded_videos or a.mjpeg_videos):
+            data = video_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, cfg, rank, world, a.crop_size,
+                                      a.mjpeg_videos, a.dct_method)
         else:
             data = (file_clip_batches(items, gbatch, steps, 1111 + 7919 * epoch, rank, world) if items is not None
                     else synthetic_clip_batches(steps, batch, T, S, cfg.NETWORK.NUM_CLASSES,
@@ -282,6 +291,8 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
             vpb = max(cfg.TEST.BATCH_SIZE // num_preds, 1)
             if a.use_tfrecord:
                 val = tfrecord_batches(val_items[lo:hi], vpb, cfg, a.dct_method)
+            elif a.mjpeg_videos:
+                val = mjpeg_batches(val_items[lo:hi], vpb, cfg, a.dct_method)
             elif a.decoded_videos:
                 val = video_batches(val_items[lo:hi], vpb, cfg)
             else:

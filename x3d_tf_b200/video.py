@@ -24,10 +24,11 @@ The resize is TF 2.4's ResizeBilinear with half_pixel_centers (what `tf.image.re
 Parity of these rules with TensorFlow is unpinned (TensorFlow is not available to this project's
 tests); they are restated from the reference's source.
 
-Videos read from the reference's TFRecords (tfrecord.TFRecordVideo, JPEG frames) are packed by
-`pack_jpeg` instead of `pack`: the batch then carries the entropy-coded segments of the distinct
-frames and their headers' tables (EncodedFrames), and the frames are decoded on the device
-(x3d_jpeg_entropy / _idct / _color) into the packed buffer the clip kernel reads.
+Videos read from the reference's TFRecords (tfrecord.TFRecordVideo, JPEG frames) or from Motion-JPEG
+AVI files (avi.MJPEGVideo) are packed by `pack_jpeg` instead of `pack`: the batch then carries the
+entropy-coded segments of the distinct frames and their headers' tables (EncodedFrames), and the
+frames are decoded on the device (x3d_jpeg_entropy / _entropy_rst / _idct / _color) into the packed
+buffer the clip kernel reads.
 """
 from __future__ import annotations
 
@@ -183,7 +184,10 @@ class EncodedFrames:
     """The JPEG frames of a VideoBatch, on the host (pinned when a CUDA device is present):
     `data` the entropy-coded segments of the distinct frames, `frames` / `tables` their
     x3d_jpeg_frame / x3d_jpeg_tables records (raw bytes), the sizes of the device buffers the
-    three decode stages use, the IDCT (`method`, DCT_METHODS) and a name per frame for messages."""
+    three decode stages use, the IDCT (`method`, DCT_METHODS) and a name per frame for messages.
+    Frames with a restart interval (Motion-JPEG only) come last, from frame `nplain` on; their
+    entropy stage is x3d_jpeg_entropy_rst over `intervals` (x3d_jpeg_interval records, raw bytes,
+    empty for TFRecord batches)."""
     data: torch.Tensor          # [bytes] uint8
     frames: torch.Tensor        # [nframes * 64] uint8
     tables: torch.Tensor        # [ntables * 4200] uint8
@@ -195,10 +199,14 @@ class EncodedFrames:
     max_pixels: int
     method: int
     names: List[str]
+    intervals: Optional[torch.Tensor] = None   # [nintervals * 24] uint8
+    nintervals: int = 0
+    nplain: Optional[int] = None               # frames without a restart interval (None: all)
 
     @property
     def h2d_bytes(self) -> int:
-        return self.data.numel() + self.frames.numel() + self.tables.numel()
+        iv = self.intervals.numel() if self.intervals is not None else 0
+        return self.data.numel() + self.frames.numel() + self.tables.numel() + iv
 
     def decode(self, device, scratch: dict) -> Tuple[torch.Tensor, torch.Tensor]:
         """Copy to `device` and decode on the current stream into buffers kept in `scratch` (grown
@@ -221,7 +229,13 @@ class EncodedFrames:
         planes = buf("jpeg_planes", self.plane_bytes, torch.uint8)
         out = buf("frames", self.out_bytes, torch.uint8)
         status = buf("jpeg_status", self.nframes, torch.int32)
-        ops.jpeg_entropy(data, frames, tables, self.nframes, coef, status)
+        nplain = self.nframes if self.nplain is None else self.nplain
+        if nplain:
+            ops.jpeg_entropy(data, frames, tables, nplain, coef, status)
+        if self.nintervals:
+            iv = buf("jpeg_intervals", self.intervals.numel(), torch.uint8)
+            iv.copy_(self.intervals, non_blocking=True)
+            ops.jpeg_entropy_rst(data, frames, tables, iv, self.nintervals, coef, status, nplain, self.nframes)
         ops.jpeg_idct(coef, frames, tables, self.nframes, self.max_blocks, self.method, planes)
         ops.jpeg_color(planes, frames, self.nframes, self.max_pixels, out)
         return out, status
@@ -301,45 +315,78 @@ def pack(videos: Sequence[np.ndarray], plan: ClipPlan, pin: Optional[bool] = Non
 
 def pack_jpeg(videos: Sequence, plan: ClipPlan, pin: Optional[bool] = None,
               dct_method: str = "INTEGER_FAST") -> VideoBatch:
-    """`pack` for videos of JPEG frames (tfrecord.TFRecordVideo, or anything with `shape` and
-    `jpeg(f)` -> bytes): the entropy-coded segment of each distinct (video, frame) pair the plan
-    reads, once, in one buffer; a table set per distinct header; the frame descriptors and the
-    offsets of the decoded frames (16-byte aligned) that frame_off points at.  Headers are parsed
-    and checked here (jpeg.parse), so an unsupported or mis-sized frame raises ValueError naming
-    its video and frame before anything reaches the device.  `dct_method`: TF's decode_jpeg
-    names, INTEGER_FAST (its default) or INTEGER_ACCURATE."""
-    from . import jpeg as J
-    if dct_method not in DCT_METHODS:
-        raise ValueError(f"dct_method {dct_method!r}: INTEGER_FAST or INTEGER_ACCURATE")
+    """`pack` for videos of JPEG frames (tfrecord.TFRecordVideo, avi.MJPEGVideo, or anything with
+    `shape` and `jpeg(f)` -> bytes): the entropy-coded segment of each distinct (video, frame) pair
+    the plan reads, once, in one buffer; a table set per distinct header; the frame descriptors and
+    the offsets of the decoded frames (16-byte aligned) that frame_off points at.  Headers are parsed
+    and checked here (jpeg.parse; with mjpeg=True for videos whose `mjpeg` attribute is true), so an
+    unsupported or mis-sized frame raises ValueError naming its video and frame before anything
+    reaches the device.  `dct_method`: TF's decode_jpeg names, INTEGER_FAST (its default) or
+    INTEGER_ACCURATE."""
     shapes = [tuple(int(x) for x in v.shape) for v in videos]
     validate(plan, shapes)
     N, T = plan.frames.shape
     keys = plan.video[:, None] * (1 << 32) + plan.frames
     uniq, inv = np.unique(keys.reshape(-1), return_inverse=True)
-    recs = np.zeros(len(uniq), J.FRAME_DTYPE)
-    table_index, table_recs, segs, names = {}, [], [], []
-    seg_off = coef = plane = out = 0
-    max_blocks = max_pixels = 0
-    for n, k in enumerate(uniq):
-        v, f = int(k >> 32), int(k & 0xffffffff)
+    enc, out_off = encoded_frames(videos, [(int(k >> 32), int(k & 0xffffffff)) for k in uniq], pin, dct_method)
+    off = torch.from_numpy(out_off[inv].reshape(N * T).astype(np.int64))
+    desc = torch.from_numpy(np.ascontiguousarray(plan.desc, np.int32))
+    if enc.frames.is_pinned():
+        off, desc = off.pin_memory(), desc.pin_memory()
+    return VideoBatch(torch.empty(0, dtype=torch.uint8), off, desc, plan.shape, enc)
+
+
+def encoded_frames(videos: Sequence, pairs: Sequence[Tuple[int, int]], pin: Optional[bool] = None,
+                  dct_method: str = "INTEGER_FAST") -> Tuple[EncodedFrames, np.ndarray]:
+    """The EncodedFrames of the (video, frame) `pairs` (distinct), and the byte offset in the
+    decoded buffer of each pair's [H, W, 3] frame.  Frames without a restart interval come first in
+    the batch (x3d_jpeg_entropy), then those with one (an x3d_jpeg_interval per interval)."""
+    from . import jpeg as J
+    from . import _lib
+    if dct_method not in DCT_METHODS:
+        raise ValueError(f"dct_method {dct_method!r}: INTEGER_FAST or INTEGER_ACCURATE")
+    parsed = []
+    for v, f in pairs:
         name = f"{getattr(videos[v], 'name', f'video {v}')} frame {f}"
         buf = videos[v].jpeg(f)
         try:
-            fr = J.parse(buf)
+            fr = J.parse(buf, mjpeg=bool(getattr(videos[v], "mjpeg", False)))
         except ValueError as e:
             raise ValueError(f"{name}: {e}") from None
         h = fr.header
-        if (h.H, h.W) != shapes[v][1:3]:
-            raise ValueError(f"{name}: {h.H}x{h.W}, but frame 0 of its video is {shapes[v][1]}x{shapes[v][2]}")
+        shape = tuple(int(x) for x in videos[v].shape)
+        if (h.H, h.W) != shape[1:3]:
+            raise ValueError(f"{name}: {h.H}x{h.W}, but frame 0 of its video is {shape[1]}x{shape[2]}")
+        parsed.append((name, buf, fr))
+    order = sorted(range(len(parsed)), key=lambda n: parsed[n][2].header.ri != 0)     # stable
+    recs = np.zeros(len(parsed), J.FRAME_DTYPE)
+    out_off = np.zeros(len(parsed), np.int64)
+    table_index, table_recs, segs, names, ivs = {}, [], [], [], []
+    seg_off = coef = plane = out = 0
+    max_blocks = max_pixels = 0
+    nplain = 0
+    for n, p in enumerate(order):
+        name, buf, fr = parsed[p]
+        h = fr.header
         t = table_index.get(id(h))
         if t is None:
             t = table_index[id(h)] = len(table_recs)
             table_recs.append(h)
-        mcux, mcuy = -(-h.W // (8 * h.hs)), -(-h.H // (8 * h.vs))
-        blocks = mcux * mcuy * (h.hs * h.vs + 2)
+        blocks = h.mcus * (h.hs * h.vs + 2)
         recs[n] = (seg_off, coef, plane, out, fr.seg_len, h.H, h.W, h.hs, h.vs, t, n, 0)
+        if h.ri:
+            iv = np.zeros(len(fr.intervals), J.INTERVAL_DTYPE)
+            iv["off"] = fr.intervals[:, 0] - fr.seg_off + seg_off
+            iv["len"] = fr.intervals[:, 1]
+            iv["frame"] = n
+            iv["mcu0"] = np.arange(len(iv)) * h.ri
+            iv["nmcu"] = np.minimum(h.ri, h.mcus - iv["mcu0"])
+            ivs.append(iv)
+        else:
+            nplain = n + 1
         segs.append(memoryview(buf)[fr.seg_off:fr.seg_off + fr.seg_len])
         names.append(name)
+        out_off[p] = out
         seg_off += fr.seg_len
         coef += blocks
         plane += blocks * 64
@@ -354,13 +401,13 @@ def pack_jpeg(videos: Sequence, plan: ClipPlan, pin: Optional[bool] = None,
     tables = np.stack([h.tables for h in table_recs])
     frames_t = torch.from_numpy(recs.view(np.uint8).copy())
     tables_t = torch.from_numpy(tables.view(np.uint8).reshape(-1).copy())
-    off = torch.from_numpy(recs["out_off"][inv].reshape(N * T).astype(np.int64))
-    desc = torch.from_numpy(np.ascontiguousarray(plan.desc, np.int32))
+    iv = np.concatenate(ivs) if ivs else np.zeros(0, J.INTERVAL_DTYPE)
+    iv_t = torch.from_numpy(iv.view(np.uint8).copy())
     if pin:
-        frames_t, tables_t, off, desc = (t.pin_memory() for t in (frames_t, tables_t, off, desc))
-    enc = EncodedFrames(data, frames_t, tables_t, len(uniq), coef, plane, out, max_blocks, max_pixels,
-                        DCT_METHODS[dct_method], names)
-    return VideoBatch(torch.empty(0, dtype=torch.uint8), off, desc, plan.shape, enc)
+        frames_t, tables_t, iv_t = (t.pin_memory() for t in (frames_t, tables_t, iv_t))
+    enc = EncodedFrames(data, frames_t, tables_t, len(parsed), coef, plane, out, max_blocks, max_pixels,
+                        DCT_METHODS[dct_method], names, iv_t, len(iv), nplain if ivs else None)
+    return enc, out_off
 
 
 def _pack(videos, plan: ClipPlan, dct_method: str) -> VideoBatch:
