@@ -109,6 +109,16 @@ int x3d_pw_fwd(const x3d_pw_args* args, void* stream);
 int x3d_tf32_split(const float* W, float* out, int rows, int cols, int ld, int transpose, void* stream);
 int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float* bias, float* D, int64_t M, int K,
                     int Nc, int lda, int ldd, int relu, double* stats, void* stream);
+/* The same GEMM in the bf16 operand mode of the mixed-precision training step (kind::f16 MMA, fp32
+ * accumulation): D = act(bias + bf16(A) . Wb^T), A rounded to bf16 (round-to-nearest-even) in shared
+ * memory after the fp32 TMA load; arguments, constraints and the stats epilogue as x3d_pw_tf32_fwd.
+ *   Wb bf16 [Nc][round_up(K, 8)] (padding zero), produced by
+ * x3d_bf16_round(W, out, rows, cols, ld, transpose): out[r][c] = bf16_rn(W[r*ld + c]), or of
+ *   W[c*ld + r] when transpose = 1, rows of pitch round_up(cols, 8) with zero padding (orientations as
+ *   x3d_tf32_split). */
+int x3d_bf16_round(const float* W, void* out, int rows, int cols, int ld, int transpose, void* stream);
+int x3d_pw_bf16_train_fwd(const float* A, const void* Wb, const float* bias, float* D, int64_t M, int K,
+                          int Nc, int lda, int ldd, int relu, double* stats, void* stream);
 
 /* ---- Channelwise 3x3x3 convolution: Bottleneck.b + bn_b, model.py:309-310 -------------------
  * Grouped Conv3D(groups=C) stride (1,s,s), TF padding='same' (T: 1 before; H/W: pad_h/pad_w
@@ -496,6 +506,11 @@ int x3d_d2f(const double* in, float* out, int64_t n, float scale, void* stream);
  * fp64 atomics into dW either way. */
 int x3d_pw_wgrad(const float* A, const float* dD, double* dW, int64_t M, int K, int N, int lda,
                  int ldd, int gather, int Ho, int Wo, int Hi, int Wi, int stride, void* stream);
+/* The backward-filter of the mixed-precision step: dW[k,n] += sum_m bf16(A[row(m),k]) * bf16(dD[m,n])
+ * (round-to-nearest-even), mma.sync m16n8k16 bf16 with fp32 partial sums per 32-row chunk, fp64 atomics
+ * into dW.  Arguments as x3d_pw_wgrad; K, N, lda, ldd multiples of 4, A and dD 16-byte aligned. */
+int x3d_pw_wgrad_bf16(const float* A, const float* dD, double* dW, int64_t M, int K, int N, int lda,
+                      int ldd, int gather, int Ho, int Wo, int Hi, int Wi, int stride, void* stream);
 /* Backward-data / backward-filter of the channelwise 3x3x3 conv (Bottleneck.b, model.py:259-267) */
 int x3d_dw_dgrad(const float* dy, const float* w, float* dx, int N, int T, int H, int W, int C,
                  int stride, int pad_h, int pad_w, void* stream);

@@ -99,6 +99,8 @@ SIGNATURES = {
     "x3d_pw_fwd": (C.c_int, [C.POINTER(PwArgs), C.c_void_p]),
     "x3d_tf32_split": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "x3d_pw_tf32_fwd": (C.c_int, [C.c_void_p] * 4 + [C.c_int64] + [C.c_int] * 5 + [C.c_void_p, C.c_void_p]),
+    "x3d_bf16_round": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "x3d_pw_bf16_train_fwd": (C.c_int, [C.c_void_p] * 4 + [C.c_int64] + [C.c_int] * 5 + [C.c_void_p, C.c_void_p]),
     "x3d_dw_partial_blocks": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "x3d_dw3x3x3_fwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -131,6 +133,7 @@ SIGNATURES = {
     "x3d_bn_bwd_apply": (C.c_int, [C.c_void_p] * 8 + [C.c_int64, C.c_int, C.c_void_p]),
     "x3d_d2f": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p]),
     "x3d_pw_wgrad": (C.c_int, [C.c_void_p] * 3 + [C.c_int64] + [C.c_int] * 10 + [C.c_void_p]),
+    "x3d_pw_wgrad_bf16": (C.c_int, [C.c_void_p] * 3 + [C.c_int64] + [C.c_int] * 10 + [C.c_void_p]),
     "x3d_dw_dgrad": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 8 + [C.c_void_p]),
     "x3d_dw_wgrad": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 8 + [C.c_void_p]),
     "x3d_stem_convs_fwd": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 5 + [C.c_void_p]),

@@ -16,6 +16,8 @@
 //     accumulator; tcgen05.commit frees ring stages / publishes the accumulator;
 //   * 4 epilogue warps drain TMEM (tcgen05.ld), add the bias, apply ReLU and store fp32 rows through
 //     128B-swizzled staging and TMA box stores (clipped at M / Nc).
+// The same pipeline has a bf16 operand mode for the mixed-precision training step
+// (x3d_pw_bf16_train_fwd, see pw_tc_body): bf16 RNE operands, one kind::f16 MMA per K=16 step.
 #include <stdlib.h>
 
 #include "tma_common.cuh"
@@ -76,6 +78,20 @@ __device__ __forceinline__ uint32_t make_idesc_tf32(int n) {
   return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(n >> 3) << 17) |
          (static_cast<uint32_t>(kBlockM >> 4) << 24);
 }
+// The same for kind::f16 with A = B = BF16 (format code 1).
+__device__ __forceinline__ uint32_t make_idesc_bf16(int n) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) |
+         (static_cast<uint32_t>(kBlockM >> 4) << 24);
+}
+__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
+                                         uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2,
                                             uint64_t* bar) {
   asm volatile(
@@ -100,23 +116,36 @@ __device__ __forceinline__ void split_tf32(uint32_t x, uint32_t& hi, uint32_t& l
   lo = __float_as_uint(__uint_as_float(x) - __uint_as_float(hi));
 }
 
+// {lo, hi} -> one bf16x2 word (lo in the low half, the lower address), round-to-nearest-even as
+// torch's .to(torch.bfloat16)
+__device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
+  uint32_t d;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+  return d;
+}
+
 struct Params {
   const float* bias;
   double* stats;   // [2][Nc] column sums / sums of squares of D (BatchNorm batch statistics), or nullptr
   long M;
   int Nc;          // output columns
   int NT;          // N tile (multiple of 32, <= 256)
-  int KC;          // 32-wide K chunks
-  int k8_last;     // K=8 MMA steps in the last chunk (1..4)
+  int KC;          // 32-wide K chunks (bf16: 64-wide)
+  int k8_last;     // K=8 (bf16: K=16) MMA steps in the last chunk (1..4)
   int stages;      // ring depth
-  int stage_bytes; // 2 * kATile + 2 * NT * 128
+  int stage_bytes; // 2 * kATile + 2 * NT * 128 (bf16: 3 * kATile + NT * 128)
   int tmem_cols;   // power of two >= 2 * NT
   int relu;
 };
 
-__global__ void __launch_bounds__(kThreads, 1)
-pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                  const __grid_constant__ CUtensorMap tmD, const Params p) {
+// kBf16 = false: the 3xTF32 split above.  kBf16 = true: the bf16 operand mode of the mixed-precision
+// training step.  A ring stage then holds two fp32 A boxes (K columns [64kc, 64kc+32) and [+32, +64)),
+// the bf16 RNE tile of both (128 rows x 64 bf16 = one 128-byte swizzle row each, the layout
+// tcgen05.mma kind::f16 reads) and one bf16 B chunk [NT][64] (tmB 2-D over the bf16 [Nc][K] weights);
+// one MMA per K=16 step.  The epilogue is the same.
+template <bool kBf16>
+__device__ __forceinline__ void pw_tc_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmD,
+                                           const Params p) {
   extern __shared__ __align__(1024) uint8_t tf_smem_raw[];
   const uint32_t raw_s = smem_u32(tf_smem_raw);
   const uint32_t base_s = (raw_s + 1023u) & ~1023u;
@@ -179,17 +208,25 @@ pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         for (int kc = 0; kc < p.KC; ++kc) {
           mbar_wait(&empty[s], ph ^ 1);
           const uint32_t st = ring_s + s * p.stage_bytes;
-          mbar_expect_tx(&full[s], static_cast<uint32_t>(kATile + 2 * b_plane));
-          tma_load_2d_s(st, &tmA, kc * kBlockK, row0, &full[s]);
-          tma_load_3d(st + 2 * kATile, &tmB, kc * kBlockK, n0, 0, &full[s]);
-          tma_load_3d(st + 2 * kATile + b_plane, &tmB, kc * kBlockK, n0, 1, &full[s]);
+          if constexpr (kBf16) {
+            // both A boxes always: a box past K is zero-filled and still counts its bytes
+            mbar_expect_tx(&full[s], static_cast<uint32_t>(2 * kATile + b_plane));
+            tma_load_2d_s(st, &tmA, kc * 2 * kBlockK, row0, &full[s]);
+            tma_load_2d_s(st + kATile, &tmA, kc * 2 * kBlockK + kBlockK, row0, &full[s]);
+            tma_load_2d_s(st + 3 * kATile, &tmB, kc * 2 * kBlockK, n0, &full[s]);
+          } else {
+            mbar_expect_tx(&full[s], static_cast<uint32_t>(kATile + 2 * b_plane));
+            tma_load_2d_s(st, &tmA, kc * kBlockK, row0, &full[s]);
+            tma_load_3d(st + 2 * kATile, &tmB, kc * kBlockK, n0, 0, &full[s]);
+            tma_load_3d(st + 2 * kATile + b_plane, &tmB, kc * kBlockK, n0, 1, &full[s]);
+          }
           if (++s == p.stages) { s = 0; ph ^= 1; }
         }
       }
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
-    const uint32_t idesc = make_idesc_tf32(p.NT);
+    const uint32_t idesc = kBf16 ? make_idesc_bf16(p.NT) : make_idesc_tf32(p.NT);
     int s = 0;
     uint32_t ph = 0;
     long it = 0;
@@ -202,7 +239,18 @@ pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       for (int kc = 0; kc < p.KC; ++kc) {
         mbar_wait(&xform[s], ph);
         tcgen05_after_sync();
-        if (elect_one()) {
+        if constexpr (kBf16) {
+          if (elect_one()) {
+            const uint32_t a_bf = ring_s + s * p.stage_bytes + 2 * kATile, b_bf = a_bf + kATile;
+            const int nk = (kc == p.KC - 1) ? p.k8_last : 4;
+            for (int k = 0; k < nk; ++k) {
+              const uint32_t o = k * 32;                       // 16 bf16 = 32 bytes per K step
+              umma_f16(d_tmem, make_desc_sw128(a_bf + o), make_desc_sw128(b_bf + o), idesc, (kc | k) != 0 ? 1u : 0u);
+            }
+            umma_commit(&empty[s]);
+            if (kc == p.KC - 1) umma_commit(&t_full[as]);
+          }
+        } else if (elect_one()) {
           const uint32_t a_hi = ring_s + s * p.stage_bytes, a_lo = a_hi + kATile;
           const uint32_t b_hi = a_hi + 2 * kATile, b_lo = b_hi + b_plane;
           const int nk = (kc == p.KC - 1) ? p.k8_last : 4;
@@ -317,6 +365,28 @@ pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     for (long tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
       for (int kc = 0; kc < p.KC; ++kc) {
         mbar_wait(&full[s], ph);
+        if constexpr (kBf16) {
+          // 16-byte bf16 chunk e = (row r, K columns 8c..8c+8) from the fp32 chunks 2(c%4), 2(c%4)+1 of box c/4
+          const uint32_t st = ring_s + s * p.stage_bytes;
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            const int e = tt + i * 256, r = e >> 3, c = e & 7;
+            const uint32_t x = static_cast<uint32_t>(r & 7), row = st + static_cast<uint32_t>(r) * 128;
+            const uint32_t src = row + (c >> 2) * kATile, c0 = static_cast<uint32_t>((c & 3) * 2);
+            float f[8];
+            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(f[0]), "=f"(f[1]), "=f"(f[2]), "=f"(f[3]) : "r"(src + ((c0 ^ x) << 4)));
+            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(f[4]), "=f"(f[5]), "=f"(f[6]), "=f"(f[7]) : "r"(src + (((c0 + 1) ^ x) << 4)));
+            uint32_t b[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) b[j] = pack_bf16x2_rn(f[2 * j], f[2 * j + 1]);
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(row + 2 * kATile + ((static_cast<uint32_t>(c) ^ x) << 4)),
+                         "r"(b[0]), "r"(b[1]), "r"(b[2]), "r"(b[3]) : "memory");
+          }
+          fence_proxy_async();
+          mbar_arrive(&xform[s]);
+          if (++s == p.stages) { s = 0; ph ^= 1; }
+          continue;
+        }
         const uint32_t a_hi = ring_s + s * p.stage_bytes + tt * 16;      // 16-byte vectors, any order: the
 #pragma unroll                                                           // split is element-wise
         for (int i = 0; i < 4; ++i) {
@@ -344,6 +414,18 @@ pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   }
 }
 
+__global__ void __launch_bounds__(kThreads, 1)
+pw_tf32_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                  const __grid_constant__ CUtensorMap tmD, const Params p) {
+  pw_tc_body<false>(tmA, tmB, tmD, p);
+}
+
+__global__ void __launch_bounds__(kThreads, 1)
+pw_bf16_train_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                        const __grid_constant__ CUtensorMap tmD, const Params p) {
+  pw_tc_body<true>(tmA, tmB, tmD, p);
+}
+
 // out[0][r][c] = hi(x), out[1][r][c] = lo(x) with x = transpose ? W[c][r] : W[r][c]
 __global__ void tf32_split_kernel(const float* __restrict__ W, float* __restrict__ out, int rows, int cols, int ld,
                                   int transpose) {
@@ -356,6 +438,20 @@ __global__ void tf32_split_kernel(const float* __restrict__ W, float* __restrict
     split_tf32(__float_as_uint(x), hi, lo);
     out[i] = __uint_as_float(hi);
     out[n + i] = __uint_as_float(lo);
+  }
+}
+
+// x3d_bf16_round: out[r][c] = bf16_rn(transpose ? W[c][r] : W[r][c]), rows of pitch round_up(cols, 8),
+// the padding columns zero (TMA needs 16-byte row strides).
+__global__ void bf16_round_kernel(const float* __restrict__ W, uint16_t* __restrict__ out, int rows, int cols,
+                                  int pitch, int ld, int transpose) {
+  const long n = static_cast<long>(rows) * pitch;
+  for (long i = static_cast<long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long>(gridDim.x) * blockDim.x) {
+    const int r = static_cast<int>(i / pitch), c = static_cast<int>(i - static_cast<long>(r) * pitch);
+    float x = 0.f;
+    if (c < cols) x = transpose ? W[static_cast<long>(c) * ld + r] : W[static_cast<long>(r) * ld + c];
+    out[i] = static_cast<uint16_t>(pack_bf16x2_rn(x, 0.f) & 0xffffu);
   }
 }
 
@@ -373,36 +469,51 @@ extern "C" int x3d_tf32_split(const float* W, float* out, int rows, int cols, in
   return check_launch("x3d_tf32_split");
 }
 
-extern "C" int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float* bias, float* D, int64_t M, int K,
-                               int Nc, int lda, int ldd, int relu, double* stats, void* stream) {
-  X3D_REQUIRE(A && Bsplit && D, X3D_ERR_INVALID_ARG, "x3d_pw_tf32_fwd: null pointer");
+extern "C" int x3d_bf16_round(const float* W, void* out, int rows, int cols, int ld, int transpose, void* stream) {
+  X3D_REQUIRE(W && out && rows > 0 && cols > 0 && ld > 0, X3D_ERR_INVALID_ARG, "x3d_bf16_round: bad argument");
+  X3D_REQUIRE(ld >= (transpose ? rows : cols), X3D_ERR_INVALID_ARG, "x3d_bf16_round: ld=%d too small", ld);
+  const int pitch = (cols + 7) / 8 * 8;
+  const long n = (long)rows * pitch;
+  long blocks = (n + 255) / 256;
+  if (blocks > 1184) blocks = 1184;
+  tf32tc::bf16_round_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      W, static_cast<uint16_t*>(out), rows, cols, pitch, ld, transpose);
+  return check_launch("x3d_bf16_round");
+}
+
+// Shared host side of both operand modes.  bf16: B is bf16 [Nc][round_up(K, 8)] from x3d_bf16_round;
+// otherwise the two fp32 planes [2][Nc][K] of x3d_tf32_split.
+static int pw_tc_launch(const char* fn, bool bf16, const float* A, const void* B, const float* bias, float* D,
+                        int64_t M, int K, int Nc, int lda, int ldd, int relu, double* stats, void* stream) {
+  X3D_REQUIRE(A && B && D, X3D_ERR_INVALID_ARG, "%s: null pointer", fn);
   X3D_REQUIRE(!stats || (!bias && !relu), X3D_ERR_INVALID_ARG,
-              "x3d_pw_tf32_fwd: column statistics are those of the plain product (no bias, no ReLU)");
-  X3D_REQUIRE(M > 0 && M < (1L << 31), X3D_ERR_INVALID_ARG, "x3d_pw_tf32_fwd: M out of range");
+              "%s: column statistics are those of the plain product (no bias, no ReLU)", fn);
+  X3D_REQUIRE(M > 0 && M < (1L << 31), X3D_ERR_INVALID_ARG, "%s: M out of range", fn);
   X3D_REQUIRE(K > 0 && K % 4 == 0 && lda % 4 == 0 && lda >= K, X3D_ERR_INVALID_ARG,
-              "x3d_pw_tf32_fwd: K=%d / lda=%d must be multiples of 4", K, lda);
+              "%s: K=%d / lda=%d must be multiples of 4", fn, K, lda);
   X3D_REQUIRE(Nc > 0 && Nc % 4 == 0 && ldd % 4 == 0 && ldd >= Nc, X3D_ERR_INVALID_ARG,
-              "x3d_pw_tf32_fwd: Nc=%d / ldd=%d must be multiples of 4", Nc, ldd);
-  X3D_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(Bsplit) & 15) == 0 &&
-              (reinterpret_cast<uintptr_t>(D) & 15) == 0, X3D_ERR_INVALID_ARG, "x3d_pw_tf32_fwd: pointers must be 16-byte aligned");
-  X3D_REQUIRE(device_sm_count() > 0 && device_is_sm100(), X3D_ERR_NO_DEVICE, "x3d_pw_tf32_fwd: needs an sm_100 device");
+              "%s: Nc=%d / ldd=%d must be multiples of 4", fn, Nc, ldd);
+  X3D_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0 &&
+              (reinterpret_cast<uintptr_t>(D) & 15) == 0, X3D_ERR_INVALID_ARG, "%s: pointers must be 16-byte aligned", fn);
+  X3D_REQUIRE(device_sm_count() > 0 && device_is_sm100(), X3D_ERR_NO_DEVICE, "%s: needs an sm_100 device", fn);
   EncodeTiledFn enc = tensor_map_encoder();
-  X3D_REQUIRE(enc != nullptr, X3D_ERR_NO_DEVICE, "x3d_pw_tf32_fwd: cuTensorMapEncodeTiled unavailable");
+  X3D_REQUIRE(enc != nullptr, X3D_ERR_NO_DEVICE, "%s: cuTensorMapEncodeTiled unavailable", fn);
 
   // N tiling: one tile up to 256 columns, else the fewest tiles of a multiple of 32 columns
   int n_tiles = (Nc + 255) / 256;
   int NT = ((Nc + n_tiles - 1) / n_tiles + 31) / 32 * 32;
   n_tiles = (Nc + NT - 1) / NT;
-  const int KC = (K + 31) / 32;
-  const int k8_last = ((K - (KC - 1) * 32) + 7) / 8;
-  const int stage_bytes = 2 * tf32tc::kATile + 2 * NT * 128;
+  const int kchunk = bf16 ? 2 * tf32tc::kBlockK : tf32tc::kBlockK, kstep = bf16 ? 16 : 8;
+  const int KC = (K + kchunk - 1) / kchunk;
+  const int k8_last = ((K - (KC - 1) * kchunk) + kstep - 1) / kstep;
+  const int stage_bytes = bf16 ? 3 * tf32tc::kATile + NT * 128 : 2 * tf32tc::kATile + 2 * NT * 128;
   const int fixed = 1024 /*align*/ + 2 * tf32tc::kATile /*staging*/ + 1024 /*bias*/ + 512 /*barriers*/;
   int stages = (device_max_smem() - fixed) / stage_bytes;
-  X3D_REQUIRE(stages >= 2, X3D_ERR_UNSUPPORTED, "x3d_pw_tf32_fwd: NT=%d does not fit two ring stages", NT);
+  X3D_REQUIRE(stages >= 2, X3D_ERR_UNSUPPORTED, "%s: NT=%d does not fit two ring stages", fn, NT);
   if (stages > 4) stages = 4;
   int tmem_cols = 32;
   while (tmem_cols < 2 * NT) tmem_cols *= 2;
-  X3D_REQUIRE(tmem_cols <= 512, X3D_ERR_UNSUPPORTED, "x3d_pw_tf32_fwd: NT=%d needs too much TMEM", NT);
+  X3D_REQUIRE(tmem_cols <= 512, X3D_ERR_UNSUPPORTED, "%s: NT=%d needs too much TMEM", fn, NT);
 
   CUtensorMap tmA, tmB, tmD;
   cuuint32_t estr[3] = {1, 1, 1};
@@ -413,16 +524,24 @@ extern "C" int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float*
     CUresult r = enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(A), dims, strides, box, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "x3d_pw_tf32_fwd: tensor map for A failed (%d; K=%d M=%ld lda=%d)", (int)r, K, (long)M, lda);
+    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "%s: tensor map for A failed (%d; K=%d M=%ld lda=%d)", fn, (int)r, K, (long)M, lda);
   }
-  {
+  if (bf16) {
+    cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)Nc};
+    cuuint64_t strides[1] = {(cuuint64_t)((K + 7) / 8 * 8) * 2};
+    cuuint32_t box[2] = {64, (cuuint32_t)NT};
+    CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(B), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "%s: tensor map for B failed (%d; K=%d Nc=%d NT=%d)", fn, (int)r, K, Nc, NT);
+  } else {
     cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)Nc, 2};
     cuuint64_t strides[2] = {(cuuint64_t)K * 4, (cuuint64_t)K * 4 * (cuuint64_t)Nc};
     cuuint32_t box[3] = {32, (cuuint32_t)NT, 1};
-    CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(Bsplit), dims, strides, box, estr,
+    CUresult r = enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(B), dims, strides, box, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "x3d_pw_tf32_fwd: tensor map for B failed (%d; K=%d Nc=%d NT=%d)", (int)r, K, Nc, NT);
+    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "%s: tensor map for B failed (%d; K=%d Nc=%d NT=%d)", fn, (int)r, K, Nc, NT);
   }
   {
     cuuint64_t dims[2] = {(cuuint64_t)Nc, (cuuint64_t)M};
@@ -431,7 +550,7 @@ extern "C" int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float*
     CUresult r = enc(&tmD, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, D, dims, strides, box, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "x3d_pw_tf32_fwd: tensor map for D failed (%d; Nc=%d M=%ld ldd=%d)", (int)r, Nc, (long)M, ldd);
+    X3D_REQUIRE(r == CUDA_SUCCESS, X3D_ERR_LAUNCH, "%s: tensor map for D failed (%d; Nc=%d M=%ld ldd=%d)", fn, (int)r, Nc, (long)M, ldd);
   }
   tf32tc::Params p;
   p.bias = bias; p.stats = stats; p.M = M; p.Nc = Nc; p.NT = NT; p.KC = KC; p.k8_last = k8_last; p.stages = stages;
@@ -442,9 +561,23 @@ extern "C" int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float*
   if (gx < 1) gx = 1;
   if (gx > num_tiles) gx = (int)num_tiles;
   dim3 grid(gx, n_tiles);
-  static SmemOptIn optin;
-  const cudaError_t e = ensure_dynamic_smem(tf32tc::pw_tf32_tc_kernel, optin, smem, false);
-  X3D_REQUIRE(e == cudaSuccess, X3D_ERR_LAUNCH, "x3d_pw_tf32_fwd: smem attribute: %s", cudaGetErrorString(e));
-  tf32tc::pw_tf32_tc_kernel<<<grid, tf32tc::kThreads, smem, static_cast<cudaStream_t>(stream)>>>(tmA, tmB, tmD, p);
-  return check_launch("x3d_pw_tf32_fwd");
+  static SmemOptIn optin_tf32, optin_bf16;
+  const cudaError_t e = bf16 ? ensure_dynamic_smem(tf32tc::pw_bf16_train_tc_kernel, optin_bf16, smem, false)
+                             : ensure_dynamic_smem(tf32tc::pw_tf32_tc_kernel, optin_tf32, smem, false);
+  X3D_REQUIRE(e == cudaSuccess, X3D_ERR_LAUNCH, "%s: smem attribute: %s", fn, cudaGetErrorString(e));
+  if (bf16)
+    tf32tc::pw_bf16_train_tc_kernel<<<grid, tf32tc::kThreads, smem, static_cast<cudaStream_t>(stream)>>>(tmA, tmB, tmD, p);
+  else
+    tf32tc::pw_tf32_tc_kernel<<<grid, tf32tc::kThreads, smem, static_cast<cudaStream_t>(stream)>>>(tmA, tmB, tmD, p);
+  return check_launch(fn);
+}
+
+extern "C" int x3d_pw_tf32_fwd(const float* A, const float* Bsplit, const float* bias, float* D, int64_t M, int K,
+                               int Nc, int lda, int ldd, int relu, double* stats, void* stream) {
+  return pw_tc_launch("x3d_pw_tf32_fwd", false, A, Bsplit, bias, D, M, K, Nc, lda, ldd, relu, stats, stream);
+}
+
+extern "C" int x3d_pw_bf16_train_fwd(const float* A, const void* Wb, const float* bias, float* D, int64_t M, int K,
+                                     int Nc, int lda, int ldd, int relu, double* stats, void* stream) {
+  return pw_tc_launch("x3d_pw_bf16_train_fwd", true, A, Wb, bias, D, M, K, Nc, lda, ldd, relu, stats, stream);
 }

@@ -417,6 +417,138 @@ pw_wgrad_tf32x3_kernel(const float* __restrict__ A, const float* __restrict__ dD
       }
 }
 
+// The backward-filter of the mixed-precision step: the structure of pw_wgrad_tf32x3_kernel (same tiles,
+// warp grid, double-buffered 32-row chunks and fp32 fold per chunk, fp64 atomics), with the operands
+// rounded to bf16 (RNE, cvt.rn.bf16x2) and one m16n8k16 bf16 MMA where the 3xTF32 split issues three
+// per k8 step.  The MMA's reduction dim is the row: a register holds two consecutive rows.
+__device__ __forceinline__ uint32_t bf16x2_rn(float lo, float hi) {
+  uint32_t d;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+  return d;
+}
+__device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+      "{%0,%1,%2,%3};"
+      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
+}
+
+template <int TK, int TN>
+__global__ void __launch_bounds__(256)
+pw_wgrad_bf16_kernel(const float* __restrict__ A, const float* __restrict__ dD, double* __restrict__ dW, long M,
+                     int K, int N, int lda, int ldd, long rows_per_block, int gather, int Ho, int Wo, int Hi,
+                     int Wi, int stride) {
+  constexpr int RC = 32;
+  constexpr int WN = (TN == 64 && TK == 32) ? 8 : 4, WK = 8 / WN;
+  constexpr int MF = TK / (16 * WK), NF = TN / (8 * WN);
+  constexpr int PA = TK + 8, PD = TN + 8;
+  constexpr int VA = TK / 32, VD = TN / 32;
+  __shared__ __align__(16) float sa[2][RC][PA];
+  __shared__ __align__(16) float sd[2][RC][PD];
+  const int k0 = blockIdx.x * TK, n0 = blockIdx.y * TN;
+  const long m0 = (long)blockIdx.z * rows_per_block;
+  long m1 = m0 + rows_per_block;
+  if (m1 > M) m1 = M;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+  const int wk = (warp / WN) * MF * 16, wn = (warp % WN) * NF * 8;
+
+  float4 ra[VA], rd[VD];
+  auto fetch = [&](long mb) {
+#pragma unroll
+    for (int v = 0; v < VA; ++v) {
+      const int e = tid + v * 256, r = e / (TK / 4), k = (e % (TK / 4)) * 4;
+      const long m = mb + r;
+      ra[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (m < m1 && k0 + k < K) {
+        long arow = m;
+        if (gather) {
+          long q = m;
+          const int wo = (int)(q % Wo); q /= Wo;
+          const int ho = (int)(q % Ho); q /= Ho;
+          arow = (q * Hi + (long)ho * stride) * Wi + (long)wo * stride;
+        }
+        ra[v] = __ldg(reinterpret_cast<const float4*>(A + arow * lda + k0 + k));
+      }
+    }
+#pragma unroll
+    for (int v = 0; v < VD; ++v) {
+      const int e = tid + v * 256, r = e / (TN / 4), nn = (e % (TN / 4)) * 4;
+      const long m = mb + r;
+      rd[v] = (m < m1 && n0 + nn < N) ? __ldg(reinterpret_cast<const float4*>(dD + m * ldd + n0 + nn))
+                                      : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  };
+  auto stage = [&](int buf) {
+#pragma unroll
+    for (int v = 0; v < VA; ++v) {
+      const int e = tid + v * 256;
+      *reinterpret_cast<float4*>(&sa[buf][e / (TK / 4)][(e % (TK / 4)) * 4]) = ra[v];
+    }
+#pragma unroll
+    for (int v = 0; v < VD; ++v) {
+      const int e = tid + v * 256;
+      *reinterpret_cast<float4*>(&sd[buf][e / (TN / 4)][(e % (TN / 4)) * 4]) = rd[v];
+    }
+  };
+
+  float acc[MF][NF][4], part[MF][NF][4];
+#pragma unroll
+  for (int i = 0; i < MF; ++i)
+#pragma unroll
+    for (int j = 0; j < NF; ++j)
+#pragma unroll
+      for (int r = 0; r < 4; ++r) acc[i][j][r] = part[i][j][r] = 0.f;
+
+  fetch(m0);
+  stage(0);
+  __syncthreads();
+  int buf = 0;
+  for (long mb = m0; mb < m1; mb += RC, buf ^= 1) {
+    const bool more = mb + RC < m1;
+    if (more) fetch(mb + RC);
+#pragma unroll
+    for (int ks = 0; ks < RC; ks += 16) {
+      uint32_t a[MF][4], b[NF][2];
+#pragma unroll
+      for (int i = 0; i < MF; ++i) {
+        const float* ap = &sa[buf][ks + 2 * t][wk + i * 16 + g];
+        a[i][0] = bf16x2_rn(ap[0], ap[PA]);
+        a[i][1] = bf16x2_rn(ap[8], ap[PA + 8]);
+        a[i][2] = bf16x2_rn(ap[8 * PA], ap[9 * PA]);
+        a[i][3] = bf16x2_rn(ap[8 * PA + 8], ap[9 * PA + 8]);
+      }
+#pragma unroll
+      for (int j = 0; j < NF; ++j) {
+        const float* bp = &sd[buf][ks + 2 * t][wn + j * 8 + g];
+        b[j][0] = bf16x2_rn(bp[0], bp[PD]);
+        b[j][1] = bf16x2_rn(bp[8 * PD], bp[9 * PD]);
+      }
+#pragma unroll
+      for (int i = 0; i < MF; ++i)
+#pragma unroll
+        for (int j = 0; j < NF; ++j) mma_bf16(part[i][j], a[i], b[j]);
+    }
+#pragma unroll
+    for (int i = 0; i < MF; ++i)
+#pragma unroll
+      for (int j = 0; j < NF; ++j)
+#pragma unroll
+        for (int r = 0; r < 4; ++r) { acc[i][j][r] += part[i][j][r]; part[i][j][r] = 0.f; }
+    if (more) stage(buf ^ 1);
+    __syncthreads();
+  }
+#pragma unroll
+  for (int i = 0; i < MF; ++i)
+#pragma unroll
+    for (int j = 0; j < NF; ++j)
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int k = k0 + wk + i * 16 + g + (r >> 1) * 8, nn = n0 + wn + j * 8 + 2 * t + (r & 1);
+        if (k < K && nn < N) atomicAdd(dW + (long)k * N + nn, (double)acc[i][j][r]);
+      }
+}
+
 // ---------------------------------------------------------------- channelwise 3x3x3 backward
 // backward-data (gather form): dx[n,t,h,w,c] = sum_taps dy[n, t+1-dt, (h+ph-dh)/s, (w+pw-dw)/s, c] * w[tap,c]
 __global__ void __launch_bounds__(256)
@@ -1271,20 +1403,26 @@ int x3d_d2f(const double* in, float* out, int64_t n, float scale, void* stream) 
   return check_launch("x3d_d2f");
 }
 
-int x3d_pw_wgrad(const float* A, const float* dD, double* dW, int64_t M, int K, int N, int lda, int ldd, int gather,
-                 int Ho, int Wo, int Hi, int Wi, int stride, void* stream) {
-  X3D_REQUIRE(A && dD && dW && M > 0 && K > 0 && N > 0, X3D_ERR_INVALID_ARG, "x3d_pw_wgrad: bad argument");
-  const bool k64 = K > 32, n64 = N > 32;
+// Grid of the backward-filter kernels: TK x TN tiles of dW times row blocks of a multiple of 32 rows.
+static dim3 pw_wgrad_grid(int64_t M, int K, int N, bool k64, bool n64, long& rpb) {
   const int TK = k64 ? 64 : 32, TN = n64 ? 64 : 32;
   const long tiles = (long)((K + TK - 1) / TK) * ((N + TN - 1) / TN);
   // enough row blocks for ~8 blocks per SM in total, at least 256 rows each
   long zb = (148L * 8 + tiles - 1) / tiles;
-  long rpb = (M + zb - 1) / zb;
+  rpb = (M + zb - 1) / zb;
   if (rpb < 256) rpb = 256;
   rpb = (rpb + 31) / 32 * 32;
   zb = (M + rpb - 1) / rpb;
   if (zb > 65535) { rpb = ((M + 65534) / 65535 + 31) / 32 * 32; zb = (M + rpb - 1) / rpb; }
-  dim3 grid((K + TK - 1) / TK, (N + TN - 1) / TN, (unsigned)zb);
+  return dim3((K + TK - 1) / TK, (N + TN - 1) / TN, (unsigned)zb);
+}
+
+int x3d_pw_wgrad(const float* A, const float* dD, double* dW, int64_t M, int K, int N, int lda, int ldd, int gather,
+                 int Ho, int Wo, int Hi, int Wi, int stride, void* stream) {
+  X3D_REQUIRE(A && dD && dW && M > 0 && K > 0 && N > 0, X3D_ERR_INVALID_ARG, "x3d_pw_wgrad: bad argument");
+  const bool k64 = K > 32, n64 = N > 32;
+  long rpb;
+  const dim3 grid = pw_wgrad_grid(M, K, N, k64, n64, rpb);
 #define X3D_WG(TKK, TNN) train::pw_wgrad_kernel<TKK, TNN><<<grid, 256, 0, S(stream)>>>(A, dD, dW, M, K, N, lda, ldd, rpb, gather, Ho, Wo, Hi, Wi, stride)
 #define X3D_WGT(TKK, TNN) train::pw_wgrad_tf32x3_kernel<TKK, TNN><<<grid, 256, 0, S(stream)>>>(A, dD, dW, M, K, N, lda, ldd, rpb, gather, Ho, Wo, Hi, Wi, stride)
   const bool vec = K % 4 == 0 && N % 4 == 0 && lda % 4 == 0 && ldd % 4 == 0 &&
@@ -1303,6 +1441,27 @@ int x3d_pw_wgrad(const float* A, const float* dD, double* dW, int64_t M, int K, 
 #undef X3D_WGT
 #undef X3D_WG
   return check_launch("x3d_pw_wgrad");
+}
+
+int x3d_pw_wgrad_bf16(const float* A, const float* dD, double* dW, int64_t M, int K, int N, int lda, int ldd,
+                      int gather, int Ho, int Wo, int Hi, int Wi, int stride, void* stream) {
+  X3D_REQUIRE(A && dD && dW && M > 0 && K > 0 && N > 0, X3D_ERR_INVALID_ARG, "x3d_pw_wgrad_bf16: bad argument");
+  X3D_REQUIRE(K % 4 == 0 && N % 4 == 0 && lda % 4 == 0 && ldd % 4 == 0 && lda >= K && ldd >= N,
+              X3D_ERR_INVALID_ARG, "x3d_pw_wgrad_bf16: K=%d N=%d lda=%d ldd=%d must be multiples of 4", K, N, lda, ldd);
+  X3D_REQUIRE(reinterpret_cast<uintptr_t>(A) % 16 == 0 && reinterpret_cast<uintptr_t>(dD) % 16 == 0,
+              X3D_ERR_INVALID_ARG, "x3d_pw_wgrad_bf16: A and dD must be 16-byte aligned");
+  X3D_REQUIRE(!gather || (Ho > 0 && Wo > 0 && Hi > 0 && Wi > 0 && stride > 0), X3D_ERR_INVALID_ARG,
+              "x3d_pw_wgrad_bf16: bad gather geometry");
+  const bool k64 = K > 32, n64 = N > 32;
+  long rpb;
+  const dim3 grid = pw_wgrad_grid(M, K, N, k64, n64, rpb);
+#define X3D_WGB(TKK, TNN) train::pw_wgrad_bf16_kernel<TKK, TNN><<<grid, 256, 0, S(stream)>>>(A, dD, dW, M, K, N, lda, ldd, rpb, gather, Ho, Wo, Hi, Wi, stride)
+  if (k64 && n64) X3D_WGB(64, 64);
+  else if (k64) X3D_WGB(64, 32);
+  else if (n64) X3D_WGB(32, 64);
+  else X3D_WGB(32, 32);
+#undef X3D_WGB
+  return check_launch("x3d_pw_wgrad_bf16");
 }
 
 int x3d_dw_dgrad(const float* dy, const float* w, float* dx, int N, int T, int H, int W, int C, int stride, int pad_h,

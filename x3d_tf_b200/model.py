@@ -852,17 +852,28 @@ class X3D(Layer):
         return self.call(x, training=training, copy=copy)
 
     # ---- training mode behind the class API (train.py:128-152)
-    def _trainer(self):
+    def _trainer(self, precision: Optional[str] = None):
         """The training engine for this model's variables (training.X3DTrainer: batch-statistics BN,
         dropout, backward kernels, gradient exchange, optimizer), created on first use from the
-        current variables; `_sync_from_trainer` copies trained values back into them."""
+        current variables; `_sync_from_trainer` copies trained values back into them.  `precision`
+        ('float32' / 'mixed_bfloat16', None: the existing engine's, else float32): an engine of another
+        policy is synced back and replaced (its optimizer slots restart at zero)."""
+        tr = getattr(self, "_tr", None)
+        if tr is not None and precision is not None and tr.precision != precision:
+            self._syncing = True
+            try:
+                self._sync_from_trainer()
+            finally:
+                self._syncing = False
+            self._tr = None
         if getattr(self, "_tr", None) is None:
             import torch.distributed as dist
             from .training import X3DTrainer
             world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
             rank = dist.get_rank() if world > 1 else 0
             dev = self._device or torch.device("cuda", torch.cuda.current_device())
-            self._tr = X3DTrainer(self.cfg, device=dev, world=world, rank=rank).load(dict(self.named_variables()))
+            self._tr = X3DTrainer(self.cfg, device=dev, world=world, rank=rank,
+                                  precision=precision or "float32").load(dict(self.named_variables()))
         return self._tr
 
     def _sync_from_trainer(self):
@@ -877,17 +888,20 @@ class X3D(Layer):
         return missing
 
     def fit(self, dataset, epochs: int = 1, initial_epoch: int = 0, steps_per_epoch: Optional[int] = None,
-            lr_schedule=None, verbose: int = 0, **_):
+            lr_schedule=None, verbose: int = 0, mixed_precision: bool = False, **_):
         """Keras `model.fit` as train.py:145-152 uses it: for every epoch the learning rate comes from
         `lr_schedule(epoch)` (train.py:114-125, default training.lr_schedule of this model's cfg),
         `steps_per_epoch` batches `(clips, labels)` are taken from `dataset` (re-iterated per epoch; clips
         as for `call`, or a video.VideoBatch whose clips are built on the device),
         each one forward + backward + gradient all-reduce over the initialised torch.distributed
         group + optimizer step (cfg.TRAIN.OPTIMIZER).  Returns {"loss": [per-epoch mean]}.  The model's
-        variables hold the trained values afterwards (call / evaluate / save_weights see them)."""
+        variables hold the trained values afterwards (call / evaluate / save_weights see them).
+        `mixed_precision`: train under the 'mixed_bfloat16' policy (runtime.get_precision, as
+        train.py --mixed_precision does)."""
         from . import ops
+        from .runtime import get_precision
         from .training import lr_schedule as default_schedule
-        tr = self._trainer()
+        tr = self._trainer(get_precision(mixed_precision))
         sched = lr_schedule or (lambda e: default_schedule(self.cfg, e))
         dev = tr.device
         mean, std = tuple(self.cfg.DATA.MEAN), tuple(self.cfg.DATA.STD)

@@ -509,6 +509,60 @@ def pw_tf32(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = Non
     return out
 
 
+def bf16_round(w: torch.Tensor, *, transpose_w: bool = True) -> torch.Tensor:
+    """The stored [K, N] fp32 kernel `w` rounded to bf16 (round-to-nearest-even) in the orientation
+    `pw_bf16_train` reads: [N, round_up(K, 8)] for the forward (transpose_w=True), [K, round_up(N, 8)]
+    for backward-data; padding columns are zero."""
+    _req(w, "w")
+    if w.dtype != torch.float32 or w.dim() != 2:
+        raise TypeError("bf16_round needs a 2-D fp32 kernel")
+    K, N = w.shape
+    red, nout = (K, N) if transpose_w else (N, K)
+    out = torch.empty((nout, (red + 7) // 8 * 8), dtype=torch.bfloat16, device=w.device)
+    _launch("x3d_bf16_round", lambda: lib().x3d_bf16_round(w.data_ptr(), out.data_ptr(), nout, red, N,
+                                                         1 if transpose_w else 0, _stream()))
+    return out
+
+
+def pw_bf16_train(a: torch.Tensor, wb: torch.Tensor, red: int, bias: Optional[torch.Tensor] = None, *,
+                  relu: bool = False, M: Optional[int] = None, stats: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Pointwise conv of the mixed-precision training step (x3d_pw_bf16_train_fwd): D[M, nout] =
+    bf16(a[M, red]) . wb^T with fp32 accumulation, `wb` from `bf16_round` ([nout, round_up(red, 8)]).
+    `stats` as in `pw_tf32`."""
+    _req(a, "a")
+    _req(wb, "wb")
+    if a.dtype != torch.float32 or wb.dtype != torch.bfloat16:
+        raise TypeError("pw_bf16_train needs fp32 activations and a bf16 kernel")
+    nout = wb.shape[0]
+    if wb.shape[1] != (red + 7) // 8 * 8:
+        raise ValueError(f"wb has {wb.shape[1]} columns, expected round_up({red}, 8)")
+    M = a.shape[0] if M is None else M
+    lda = a.shape[-1]
+    if lda < red:
+        raise ValueError(f"a has {lda} columns, the reduction needs {red}")
+    out = torch.empty((M, nout), dtype=torch.float32, device=a.device)
+    _launch("x3d_pw_bf16_train_fwd", lambda: lib().x3d_pw_bf16_train_fwd(
+        a.data_ptr(), wb.data_ptr(), _ptr(bias), out.data_ptr(), M, red, nout, lda, nout, 1 if relu else 0,
+        _ptr(stats), _stream()))
+    return out
+
+
+def pw_wgrad_bf16(a: torch.Tensor, dy: torch.Tensor, dw64: torch.Tensor, *, M: Optional[int] = None,
+                  gather: Optional[Tuple[int, int, int, int, int, int]] = None) -> None:
+    """dw64[K, N] += bf16(a)^T . bf16(dy) (x3d_pw_wgrad_bf16); `gather` = (T, Ho, Wo, Hi, Wi, stride)
+    reads the rows of the strided shortcut from the full-resolution `a`."""
+    for t, n in ((a, "a"), (dy, "dy"), (dw64, "dw64")):
+        _req(t, n)
+    if a.dtype != torch.float32 or dy.dtype != torch.float32 or dw64.dtype != torch.float64:
+        raise TypeError("pw_wgrad_bf16 needs fp32 a / dy and an fp64 dw64")
+    K, N = dw64.shape
+    M = dy.shape[0] if M is None else M
+    g = gather or (0, 0, 0, 0, 0, 1)
+    _launch("x3d_pw_wgrad_bf16", lambda: lib().x3d_pw_wgrad_bf16(
+        a.data_ptr(), dy.data_ptr(), dw64.data_ptr(), M, K, N, a.shape[-1], dy.shape[-1], int(gather is not None),
+        g[1], g[2], g[3], g[4], g[5], _stream()))
+
+
 def expand_dw2_supported(T: int, H: int, W: int, cin: int, c: int, stride: int) -> int:
     """SE partial blocks per clip of the persistent fused kernel's plan, 0 if no tile plan fits."""
     return int(lib().x3d_expand_dw2_partial_blocks(T, H, W, cin, c, stride))

@@ -160,7 +160,7 @@ def synthetic_clip_batches(steps: int, batch: int, T: int, S: int, num_classes: 
                rng.integers(0, num_classes, size=batch).astype(np.int32))
 
 
-def run(argv: Optional[List[str]] = None) -> Optional[dict]:
+def build_parser() -> argparse.ArgumentParser:
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("--config", required=True, help="config .yaml (reference layout) or a variant name")
     ap.add_argument("--train_file_pattern", default=None)
@@ -182,8 +182,14 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     ap.add_argument("--batch_size", type=int, default=0, help="override cfg.TRAIN.BATCH_SIZE (global batch)")
     ap.add_argument("--crop_size", type=int, default=0, help="override cfg.DATA.TRAIN_CROP_SIZE (synthetic data)")
     ap.add_argument("--mixed_precision", action="store_true",
-                    help="train.py:26,72-74,99-100.  Not built: the training kernels compute in fp32 (the "
-                         "reference's default precision); the flag is rejected rather than ignored")
+                    help="train.py:26,72-74,99-100: the 'mixed_bfloat16' policy -- every 1x1x1 conv and Dense "
+                         "layer multiplies bf16 operands with fp32 accumulation (BatchNorm, softmax, the master "
+                         "weights and the optimizer stay fp32); validation runs the bf16 inference engine")
+    return ap
+
+
+def run(argv: Optional[List[str]] = None) -> Optional[dict]:
+    ap = build_parser()
     a = ap.parse_args(argv)
     if not a.train_file_pattern and not a.synthetic:
         ap.error("one of --train_file_pattern / --synthetic is required")
@@ -193,9 +199,6 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
         cfg = get_default_config(); cfg.merge_from_file(a.config); cfg.freeze()
     else:
         cfg = get_config(a.config)
-    if a.mixed_precision:
-        raise NotImplementedError("--mixed_precision: the training step runs in fp32 only (no 16-bit backward "
-                                  "kernels, no loss scaling); evaluation has the 16-bit policy (eval --mixed_precision)")
     if cfg.TRAIN.OPTIMIZER.lower() not in ("sgd", "adam"):
         raise NotImplementedError(f"{cfg.TRAIN.OPTIMIZER} not supported")          # train.py:96-97
     os.makedirs(a.model_dir, exist_ok=True)
@@ -219,7 +222,9 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
     from .eval import file_batches, mjpeg_batches, tfrecord_batches, tfrecord_files, video_batches
     from .video import VideoBatch
 
-    tr = X3DTrainer(cfg, device=dev, world=world, rank=rank)
+    from .runtime import get_precision, policy_dtype
+    precision = get_precision(a.mixed_precision)
+    tr = X3DTrainer(cfg, device=dev, world=world, rank=rank, precision=precision)
     # a from-scratch run starts where `X3D(cfg)` starts in the reference (train.py:128): Keras default
     # initialisers -- Glorot-uniform kernels, zero biases, BN gamma=1 / beta=0 / mean=0 / variance=1
     tr.load(keras_default_weights(cfg, seed=1111))
@@ -279,11 +284,11 @@ def run(argv: Optional[List[str]] = None) -> Optional[dict]:
             dist.all_reduce(stats)
             from .exchange import average_
             average_(tr.moving.values(), world)                              # SURVEY 8e: average at save time
-        log = {"epoch": epoch + 1, "lr": lr, "loss": float(stats[0] / max(float(stats[1]), 1.0)),
+        log = {"epoch": epoch + 1, "policy": precision, "lr": lr, "loss": float(stats[0] / max(float(stats[1]), 1.0)),
                "steps": n, "seconds": time.time() - t0}
         if val_items is not None:
             reset_block_counters()
-            m = X3D(cfg, dtype="float32").compile()
+            m = X3D(cfg, dtype=policy_dtype(precision)).compile()
             m.set_weights_dict(tr.weights())
             num_preds = cfg.TEST.NUM_TEMPORAL_VIEWS * cfg.TEST.NUM_SPATIAL_CROPS
             from .shard import shard_range

@@ -13,6 +13,12 @@ training=True; SURVEY.md Appendix A.7) with hand-written CUDA kernels behind the
 PyTorch owns device memory, the stream and the NCCL communicator; all arithmetic is in the kernels.
 fp32 activations (the reference's default precision).  First correct version: kernels are simple
 and unfused (DESIGN.md section 9).
+
+precision="mixed_bfloat16" (train.py --mixed_precision): every 1x1x1 conv and Dense layer multiplies
+bf16 operands (round-to-nearest-even) with fp32 accumulation -- forward, backward-data and
+backward-filter; activations, BatchNorm, the channelwise and stem convs, SE, softmax, the fp32 master
+weights, the fp64 gradient accumulators, the optimizers and the all-reduce stay as in float32.  bf16
+has fp32's exponent range, so no loss scaling.
 """
 from __future__ import annotations
 
@@ -64,7 +70,15 @@ def _mix64(z: int) -> int:
 class X3DTrainer:
     """`X3DTrainer(cfg).load(weights)`; `loss = trainer.step(clips, labels, lr)`."""
 
-    def __init__(self, cfg, device=None, world: int = 1, process_group=None, seed: int = 1111, rank: int = 0):
+    PRECISIONS = ("float32", "mixed_bfloat16")
+
+    def __init__(self, cfg, device=None, world: int = 1, process_group=None, seed: int = 1111, rank: int = 0,
+                 precision: str = "float32"):
+        if precision not in self.PRECISIONS:
+            raise ValueError(f"precision {precision!r}: expected one of {self.PRECISIONS}")
+        self.precision = precision
+        self.mixed = precision == "mixed_bfloat16"
+        self._wb: Dict[Tuple[int, bool], torch.Tensor] = {}     # bf16 kernels of this step (mixed)
         self.cfg = cfg
         self.rank = rank                    # mixed into the dropout stream: replicas draw independent masks
         self.arch = A.build_arch(cfg)
@@ -87,6 +101,8 @@ class X3DTrainer:
         self.gemm = _os.environ.get("X3D_TRAIN_GEMM", "tcgen05")
         self.fixed_dropout_mask: Optional[torch.Tensor] = None      # tests inject a mask
         self.relu_masks: Optional[list] = None                      # tests: record every ReLU's sign pattern
+        self.gemm_operands: Optional[dict] = None                   # tests (mixed): record every GEMM's fp32
+        #                                                             activation operand, by (pass, kernel ptr)
         ar = self.arch
         self.layout = _Arena()
         self.tf_shape: Dict[str, Tuple[int, ...]] = {}
@@ -278,10 +294,26 @@ class X3DTrainer:
         return st
 
     # ------------------------------------------------------------------ primitive ops
+    def _bf16_kernel(self, w, transpose_w):
+        """`w` rounded to bf16 in the orientation the GEMM reads, once per step: the cache is emptied when
+        a step starts, i.e. after the previous update."""
+        key = (w.data_ptr(), transpose_w)
+        if key not in self._wb:
+            self._wb[key] = ops.bf16_round(w, transpose_w=transpose_w)
+        return self._wb[key]
+
     def _pw(self, x2d, w, bias=None, relu=False, gather=None, M=None, stats=None):
         """`stats`: None, or a zeroed fp64 [2, N] slice that the GEMM epilogue fills with the column sums /
         sums of squares of the result (the following BatchNorm's batch statistics); returns (y, filled)."""
         K, N = w.shape
+        if self.mixed:
+            if gather is not None:
+                T, _, _, H, W, s = gather
+                x2d = ops.gather_rows_fwd(x2d.view(-1, T, H, W, x2d.shape[-1]), s)
+            if self.gemm_operands is not None:
+                self.gemm_operands[("fwd", w.data_ptr())] = x2d.cpu().numpy()
+            y = ops.pw_bf16_train(x2d, self._bf16_kernel(w, True), K, bias, relu=relu, stats=stats)
+            return y if stats is None else (y, True)
         if gather is None and self.gemm == "tcgen05":
             # tcgen05.mma kind::tf32, 3xTF32 split (csrc/x3d_pw_tf32_tc.cu)
             y = ops.pw_tf32(x2d, w, bias, relu=relu, transpose_w=True, M=M, stats=stats)
@@ -296,6 +328,13 @@ class X3DTrainer:
         w = self.P(name)
         K, N = w.shape
         M = dy2d.shape[0]
+        if self.mixed:
+            if self.gemm_operands is not None:
+                self.gemm_operands[("bwd", w.data_ptr())] = dy2d.cpu().numpy()
+            ops.pw_wgrad_bf16(x2d, dy2d, self.G64(name), M=M, gather=gather)
+            if not need_dx:
+                return None
+            return ops.pw_bf16_train(dy2d, self._bf16_kernel(w, False), N)
         g = gather or (0, 0, 0, 0, 0, 1)
         check(lib().x3d_pw_wgrad(x2d.data_ptr(), dy2d.data_ptr(), self.G64(name).data_ptr(), M, K, N,
                                  x2d.shape[-1], N, int(gather is not None), g[1], g[2], g[3], g[4], g[5],
@@ -374,6 +413,7 @@ class X3DTrainer:
         x = clips.contiguous()
         N, T, H, W, _ = x.shape
         self.g64.zero_()
+        self._wb.clear()
         self._stat_arena.zero_()
         self._stat_used = 0
         tape: List = []                       # backward closures, each maps dy -> dx of its op
