@@ -18,11 +18,12 @@ def _p8(c):
 
 
 def _layer_shapes():
-    """(K, N, dense) of every 1x1x1 conv / Dense layer of X3D-XS and X3D-M training (device layouts)."""
+    """(K, N, dense) of every 1x1x1 conv / Dense layer of X3D-XS, -M, -L and -XL training (device layouts).
+    X3D-XL adds a 160-column N tile (N = 312) and three N tiles (N = 632)."""
     from x3d_tf_b200.arch import build_arch
     from x3d_tf_b200.config import get_config
     out = set()
-    for v in ("X3D_XS", "X3D_M"):
+    for v in ("X3D_XS", "X3D_M", "X3D_L", "X3D_XL"):
         ar = build_arch(get_config(v))
         for b in ar.blocks:
             cin, ci, co = _p8(b.cin), _p8(b.cinner), _p8(b.cout)

@@ -96,7 +96,8 @@ def test_pointwise_backward(M, K, N, gather):
 
 
 @pytest.mark.parametrize("N,T,H,W,C,stride", [(2, 4, 8, 8, 56, 1), (1, 3, 9, 13, 24, 2), (1, 4, 16, 16, 56, 2),
-                                              (1, 5, 7, 10, 112, 1), (1, 2, 23, 23, 8, 2)])
+                                              (1, 5, 7, 10, 112, 1), (1, 2, 23, 23, 8, 2),
+                                              (1, 2, 6, 6, 632, 1)])
 def test_channelwise_backward(N, T, H, W, C, stride):
     from oracle import x3d_oracle as O
     L, check = _L()
@@ -210,7 +211,9 @@ def test_softmax_xent_and_sgd():
 @pytest.mark.parametrize("M,K,N,relu,use_bias", [(1000, 24, 56, True, True), (4096, 56, 24, False, True),
                                                  (300, 432, 192, False, False), (129, 192, 432, True, True),
                                                  (64, 432, 2048, True, False), (32, 2048, 400, False, True),
-                                                 (5000, 48, 216, True, True), (12345, 216, 96, False, True)])
+                                                 (5000, 48, 216, True, True), (12345, 216, 96, False, True),
+                                                 (3000, 280, 632, True, True), (2000, 632, 280, False, True),
+                                                 (4000, 136, 312, False, False)])
 def test_pointwise_tf32x3_tcgen05(M, K, N, relu, use_bias):
     """x3d_pw_tf32_fwd (tcgen05.mma kind::tf32, 3xTF32 split) against float64: fp32-level accuracy
     (2e-5 of the output's scale, the bound of the fp32 kernels) in both orientations -- forward

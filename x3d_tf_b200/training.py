@@ -59,6 +59,27 @@ class _Arena:
         return flat[off:off + int(np.prod(shape))].view(shape)
 
 
+def channelwise_dgrad(dy5: torch.Tensor, wb: torch.Tensor, zero_b: torch.Tensor, H: int, W: int, s: int, ph: int,
+                      pw_: int) -> torch.Tensor:
+    """Backward-data of the channelwise 3x3x3 SAME conv (taps `wb` [27, C], stride (1, s, s), pads before
+    `ph`, `pw_`): dy5 [N, T, Ho, Wo, C] -> dx [N, T, H, W, C], through the forward kernel.  For stride 1 it
+    is the SAME convolution of dy with the taps reversed; for stride 2 dy is first zero-dilated onto the
+    input grid (at offset 1 - pad_before per axis), which makes it the same stride-1 convolution.
+    tests/test_gpu_train_kernels_at_scale.py checks this function against float64 autograd; x3d_dw_dgrad,
+    the direct gather form, stays in the ABI.  `zero_b`: a zero [C] bias."""
+    N, T, Ho, Wo, ci = dy5.shape
+    wflip = wb.flip(0).contiguous()
+    if s == 1:
+        g = dy5
+    else:
+        g = torch.zeros((N, T, H, W, ci), dtype=torch.float32, device=dy5.device)
+        off = ((1 - ph) * W + (1 - pw_)) * ci
+        check(lib().x3d_strided_add(dy5.data_ptr(), g.data_ptr() + 4 * off, N * T, Ho, Wo, H, W, s, ci, _s()),
+              "x3d_strided_add")
+    dx, _ = ops.dw_fwd(g, wflip, zero_b, 1, 1, 1, False)
+    return dx
+
+
 def _mix64(z: int) -> int:
     """splitmix64 finaliser (the same hash the dropout kernel applies per element)."""
     z &= (1 << 64) - 1
@@ -545,21 +566,7 @@ class X3DTrainer:
             dy5 = dy.view(N, T, Ho, Wo, ci)
             check(L.x3d_dw_wgrad(a_out.data_ptr(), dy5.data_ptr(), self.G64(q + "/b/kernel").data_ptr(), N, T, H, W,
                                  ci, s, ph, pw_, _s()), "x3d_dw_wgrad")
-            # Backward-data through the forward kernel: for stride 1 it is the SAME convolution of dy
-            # with the taps reversed; for stride 2 dy is first zero-dilated onto the input grid (at
-            # offset 1 - pad_before per axis), which makes it the same stride-1 convolution.
-            # (x3d_dw_dgrad, the direct gather form, stays in the ABI and is what the kernel test checks
-            # this against.)
-            wflip = wb.flip(0).contiguous()
-            if s == 1:
-                g = dy5
-            else:
-                g = torch.zeros((N, T, H, W, ci), dtype=torch.float32, device=x.device)
-                off = ((1 - ph) * W + (1 - pw_)) * ci
-                check(L.x3d_strided_add(dy5.data_ptr(), g.data_ptr() + 4 * off, N * T, Ho, Wo, H, W, s, ci, _s()),
-                      "x3d_strided_add")
-            dx, _ = ops.dw_fwd(g, wflip, zero_b, 1, 1, 1, False)
-            return dx.view(-1, ci)
+            return channelwise_dgrad(dy5, wb, zero_b, H, W, s, ph, pw_).view(-1, ci)
         tape.append(dw_bwd)
         b_out = self._bn_fwd(b_pre.view(-1, ci), q + "/bn_b", False, tape)
         # ---- SE (model.py:311-315) + swish (:316)
